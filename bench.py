@@ -2,6 +2,7 @@
 """bench.py -- detector-samples/s per destriper PCG iteration (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c2|c5] [--regen]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's compiled CPU path, bounded sample
 
 A *step* is one PCG iteration of the Offset-template destriper (SolverLHS.apply + the vector
@@ -86,7 +87,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the e2e MapMaker run and the other-workload sub-runs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed PCG iterations computed, after the last timed "
+                         "step, to DIR/<name>.npy (same arguments -> same inputs, so two builds "
+                         "can be compared output for output)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -494,6 +502,34 @@ def time_iterations(ds, st, sqsum_init, steps, warmup, world, lib):
         # per LHS the amplitude prescale + (pass 1, ranged reduction, pass 2) per chunk
         launches += steps * (1 + 3 * int(ds.n_chunks))
     return t0.elapsed_time(t1) / max(steps, 1), history, int(launches)
+
+
+DUMP_SAMPLE = 1 << 20   # entries per dumped vector: three vectors + their index stay below 64 MB
+
+
+def dump_outputs(out_dir, st, history, rank):
+    """What the timed PCG iterations leave a caller of Destriper.solve after the last timed step:
+    the amplitudes x, the residual r and the LHS q = A d of the new direction (float64; for longer
+    vectors a fixed, seeded sample of DUMP_SAMPLE entries, whose positions are in
+    sample_index.npy), and the relative residual of every step, warm-up included.  Ranks other
+    than 0 add a _rank<r> suffix."""
+    import torch
+
+    n = st.x.numel()
+    if n > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    else:
+        idx = np.arange(n)
+    idx_dev = torch.from_numpy(idx).to(st.x.device)
+    arrays = {"sample_index": idx.astype(np.float64),
+              "amplitudes": st.x[idx_dev].cpu().numpy(),
+              "residual": st.r[idx_dev].cpu().numpy(),
+              "lhs": st.q[idx_dev].cpu().numpy(),
+              "relative_residuals": np.asarray(history, dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if rank == 0 else f"_rank{rank}"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 def time_phases(ds, st, reps=5):
@@ -964,6 +1000,8 @@ def main_gpu(args):
     ms_step, history, launches = time_iterations(ds, st, sqsum_init, args.steps, args.warmup,
                                                  world, lib)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, st, history, rank)
 
     path, blocked = describe_path(ds, dobs, lib, args.regen, world)
     fused = blocked and world == 1 and ds.fuse_lhs and len(ds.obs) == 1

@@ -2,12 +2,19 @@ import os
 import sys
 
 import pytest
+import threadpoolctl
 
 # The reference's CPU project_signal accumulates with OpenMP atomics (template_offset.cpp:
 # 301-327): only a single-threaded oracle is deterministic / bit-comparable.
 # Forced (not setdefault): a caller's OMP_NUM_THREADS > 1 would make the bit-for-bit checks against
 # the compiled reference flaky.  TB_TEST_OMP_THREADS overrides it for experiments.
 os.environ["OMP_NUM_THREADS"] = os.environ.get("TB_TEST_OMP_THREADS", "1")
+
+# numpy's OpenBLAS splits a dot product of more than 10 000 elements into one partial sum per
+# thread, so the oracle's PCG results on the larger golden fixtures (c2/c4/c5_wide) depend on its
+# thread count: they were stored with 8 threads.  numpy is already loaded when this file runs, so
+# the count is set through the library rather than through OPENBLAS_NUM_THREADS.
+threadpoolctl.threadpool_limits(8, user_api="blas")
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:

@@ -6,8 +6,9 @@ Run in the build container (needs /root/reference compiled by oracle/build_ref.s
 
 Inputs are regenerated deterministically by toast_b200.synthetic; the committed files hold the
 outputs of the REFERENCE's compiled kernels driven by the oracle's restatement of the Python
-glue: pixels (int32, every sample), weights (every 16th sample + per-detector column sums), the
-noise-weighted map, RHS, LHS(1), amplitudes after 2 PCG iterations and the residual history.
+glue: pixels (int32, every sample), weights (every 16th sample, as the SHA-256 of those values plus
+512 of them, + per-detector column sums), the noise-weighted map, RHS, LHS(1), amplitudes after 2
+PCG iterations and the residual history.
 """
 
 import os
@@ -19,6 +20,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
+from helpers import pack_golden  # noqa: E402
 from oracle import toast_oracle as O  # noqa: E402
 from toast_b200 import synthetic as S  # noqa: E402
 
@@ -59,7 +61,7 @@ def main():
             os.path.join(HERE, f"{name}.npz"),
             workload=wl, n_det=nd, n_samp=ns, nside=nside, weight_stride=WSTRIDE,
             pixels=pb.pixels.astype(np.int32),
-            weights_strided=np.ascontiguousarray(pb.weights[:, ::WSTRIDE, :]),
+            **pack_golden(None, {"weights_strided": pb.weights[:, ::WSTRIDE, :]}),
             weights_colsum=pb.weights.sum(axis=1),
             hit_submaps=pb.hit_submaps,
             zmap_index=nz.astype(np.int32),

@@ -1,5 +1,6 @@
 """Shared helpers for the parity tests."""
 
+import hashlib
 import os
 import sys
 
@@ -13,6 +14,8 @@ from oracle import toast_oracle as O  # noqa: E402  (the checker; never the thin
 from toast_b200 import synthetic as S  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+GOLDEN_FULL_MAX = 4096   # golden arrays up to this many elements are stored whole,
+GOLDEN_SAMPLE = 512      # larger ones as a SHA-256 of their bytes plus this many sampled values
 
 # north_star tolerance: fp64 results within 1e-10 relative of the reference COMPILED path.
 # Element-wise relative error is meaningless for weights/maps that cross zero (cos 2a -> 0), so
@@ -28,6 +31,41 @@ def assert_close_norm(actual, expected, rtol=RTOL, what=""):
     err = np.max(np.abs(actual - expected)) if expected.size else 0.0
     assert np.all(np.isfinite(actual)), f"{what}: non-finite values"
     assert err <= rtol * max(scale, 1e-300), f"{what}: max|diff| {err:.3e} > {rtol:g} * {scale:.3e}"
+
+
+def digest(a):
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def _golden_sample_index(n):
+    return np.sort(np.random.default_rng(0).choice(n, GOLDEN_SAMPLE, replace=False))
+
+
+def pack_golden(prefix, arrays):
+    """The npz entries that pin ``arrays`` (name -> ndarray) bit for bit, under
+    ``prefix/name`` (or ``name`` when ``prefix`` is None)."""
+    out = {}
+    for key, a in arrays.items():
+        a = np.asarray(a)
+        name = f"{prefix}/{key}" if prefix else key
+        if a.size <= GOLDEN_FULL_MAX:
+            out[name] = a
+        else:
+            out[name + "/sha256"] = np.array(digest(a))
+            out[name + "/sample"] = a.reshape(-1)[_golden_sample_index(a.size)]
+    return out
+
+
+def assert_packed(g, name, a):
+    """``a`` is bit for bit the array that pack_golden stored as ``name`` in the npz ``g``."""
+    a = np.asarray(a)
+    if name in g.files:
+        np.testing.assert_array_equal(a, g[name], err_msg=name)
+    else:
+        np.testing.assert_array_equal(a.reshape(-1)[_golden_sample_index(a.size)],
+                                      g[name + "/sample"], err_msg=name)
+        assert digest(a) == str(g[name + "/sha256"]), name
 
 
 def checker():
