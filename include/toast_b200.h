@@ -172,6 +172,21 @@ int tb_pointing_fused(
     int64_t nside, int nest, const double *epsilon, const double *gamma, const double *cal,
     int IAU, int64_t n_det, int64_t n_samp, int mem, void *stream);
 
+/* The same fused expansion onto a flat WCS projection (f4): the pixel step is tb_pixels_wcs's, so
+ * outputs are bit-identical to tb_pointing_detector -> tb_pixels_wcs -> tb_stokes_weights_IQU.
+ * Arguments as tb_pointing_fused with the projection in place of nside / nest; the descriptor is
+ * validated as tb_pixels_wcs does, and hit_submaps (or NULL) must cover n_col * n_row pixels. */
+int tb_pointing_fused_wcs(
+    const double *focalplane /* [S] */, const double *boresight /* [L] */,
+    const uint8_t *shared_flags /* [L] or NULL */, uint8_t shared_flag_mask,
+    const int32_t *quat_index, double *quats, int64_t n_quat_buf,
+    const int32_t *pixel_index, int64_t *pixels, int64_t n_pix_buf,
+    const int32_t *weight_index, double *weights, int64_t n_w_buf,
+    const double *hwp /* [L] or NULL */, const tb_interval *intervals, int64_t n_view,
+    uint8_t *hit_submaps /* [S] or NULL */, int64_t n_submap, int64_t n_pix_submap,
+    const tb_wcs_desc *wcs, const double *epsilon, const double *gamma, const double *cal,
+    int IAU, int64_t n_det, int64_t n_samp, int mem, void *stream);
+
 /* ---- a4  noise_weight : ops_noise_weight.cpp:12-118 ------------------------------------- */
 int tb_noise_weight(
     double *det_data /* [L] [n_data_buf,n_samp] in/out */, int64_t n_data_buf,
@@ -304,6 +319,11 @@ typedef struct {
 } tb_obs_desc;
 
 tb_obs *tb_obs_create(const tb_obs_desc *desc);
+/* An observation whose pixels are those of a flat WCS projection: `nside` / `nest` of the
+ * descriptor are ignored, the projection is validated as tb_pixels_wcs does and kept for the
+ * regenerated-pointing passes (regen != 0), which then compute the pixels tb_pointing_fused_wcs
+ * stores.  Every other pass works on local pixel numbers and is the same for both kinds. */
+tb_obs *tb_obs_create_wcs(const tb_obs_desc *desc, const tb_wcs_desc *wcs);
 void tb_obs_destroy(tb_obs *obs);
 
 int tb_lhs_pass1(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_flags,

@@ -7,6 +7,7 @@
 
 #include "tb_device.cuh"
 #include "tb_runtime.cuh"
+#include "tb_wcs.cuh"
 
 using tbd::Views;
 
@@ -23,6 +24,8 @@ struct tb_obs {
     const double *gamma = nullptr;
     const double *det_scale = nullptr;
     tb_obs_desc d; // copy of the descriptor (host pointers in it are NOT kept alive)
+    int is_wcs = 0; // pixels of a flat projection (tb_obs_create_wcs): regenerated with `wcs`
+    tbw::Wcs wcs{};
     int64_t n_amp_det = 0;
     // per-interval tiles for the TMA-staged passes: [n_tiles] x {s0, off, cnt, view}
     int64_t *tiles = nullptr;

@@ -7,7 +7,7 @@
 //     traffic stays in L2,
 //   * once-used timestream data is read/written with streaming (evict-first) accesses.
 #include "tb_device.cuh"
-#include "tb_wcs.cuh"
+#include "tb_pixelise.cuh"
 #include "tb_runtime.cuh"
 
 using namespace tbd;
@@ -210,9 +210,10 @@ struct FusedOut {
     uint8_t *hsub;
 };
 
-template <bool NEST, bool HWP>
+// PIX: the pixelisation policy of tb_pixelise.cuh (HEALPix NEST / RING, or WCS)
+template <class PIX, bool HWP>
 __global__ void __launch_bounds__(kThreads, TB_POINT_CTAS)
-k_pointing_fused(Views V, int64_t n_det, int64_t n_samp, tbm::PixCtx ctx,
+k_pointing_fused(Views V, int64_t n_det, int64_t n_samp, typename PIX::Geom geom,
                  const double *__restrict__ fp, const double *__restrict__ boresight,
                  const uint8_t *__restrict__ flags, uint8_t mask, FusedOut o,
                  const double *__restrict__ hwp, const double *__restrict__ epsilon,
@@ -228,19 +229,13 @@ k_pointing_fused(Views V, int64_t n_det, int64_t n_samp, tbm::PixCtx ctx,
         tbm::Quat q = detector_quat(boresight, s, bad, f);
         if (o.quats) st_quat_stream(o.quats + ((int64_t)__ldg(o.qidx + det) * n_samp + s) * 4, q);
         if (o.pixels) {
-            double dx, dy, dz;
-            tbm::rot_zaxis(q, dx, dy, dz);
-            int ex = 0;
-            int64_t p = tbm::vec2pix<NEST>(ctx, dx, dy, dz, &ex);
-            n_exact += ex;
+            int64_t p = PIX::pixel(geom, q, n_exact);
             if (bad) {
                 p = -1;
-            } else if (o.hsub) {
+            } else if (o.hsub && (!PIX::kMayMiss || p >= 0)) {
                 // the thread's samples mostly stay in one submap: look at the mask only when
-                // the submap changes (32-bit conversions when the pixel number allows)
-                const int64_t sm = ctx.small
-                    ? (int64_t)__double2int_rz(((double)(int)p + 0.5) * inv_nps)
-                    : fast_div(p, inv_nps);
+                // the submap changes
+                const int64_t sm = PIX::submap(geom, p, inv_nps);
                 if (sm != last_sm) {
                     if (o.hsub[sm] == 0) o.hsub[sm] = 1;
                     last_sm = sm;
@@ -673,26 +668,11 @@ int tb_pixels_wcs(const tb_wcs_desc *wcs, const int32_t *quat_index, const doubl
                   void *stream) {
     TB_API_BEGIN
     tbr::Resolver R(mem, stream);
-    TB_REQUIRE(wcs != nullptr, "NULL projection");
-    TB_REQUIRE(wcs->projection >= 0 && wcs->projection <= 5, "unknown projection code");
-    TB_REQUIRE(wcs->n_col > 0 && wcs->n_row > 0, "the projection has non-positive dimensions");
-    TB_REQUIRE(wcs->cdelt[0] != 0.0 && wcs->cdelt[1] != 0.0, "CDELT must be non-zero");
-    TB_REQUIRE(hit_submaps == nullptr ||
-                   (n_pix_submap > 0 && n_submap * n_pix_submap >= wcs->n_col * wcs->n_row),
+    tbw::Wcs w = tbp::wcs_from_desc(wcs);
+    TB_REQUIRE(hit_submaps == nullptr || (n_pix_submap > 0 && n_submap * n_pix_submap >= w.n_pix),
                "hit_submaps too small for the projection");
     check_index(quat_index, n_det, n_quat_buf, "quat");
     check_index(pixel_index, n_det, n_pix_buf, "pixel");
-    tbw::Wcs w;
-    w.proj = wcs->projection;
-    for (int k = 0; k < 5; ++k) w.euler[k] = wcs->euler[k];
-    for (int k = 0; k < 2; ++k) {
-        w.crpix[k] = wcs->crpix[k];
-        w.cdelt[k] = wcs->cdelt[k];
-    }
-    w.cea_lambda = wcs->cea_lambda;
-    w.n_col = wcs->n_col;
-    w.n_pix = wcs->n_col * wcs->n_row;
-    w.is_azimuth = wcs->is_azimuth;
     Views V = make_views(R, intervals, n_view, n_samp);
     const int32_t *d_qi = R.small(quat_index, n_det);
     const int32_t *d_pi = R.small(pixel_index, n_det);
@@ -752,19 +732,23 @@ int tb_stokes_weights_I(const int32_t *weight_index, double *weights, int64_t n_
     TB_API_END
 }
 
-int tb_pointing_fused(const double *focalplane, const double *boresight,
-                      const uint8_t *shared_flags, uint8_t shared_flag_mask,
-                      const int32_t *quat_index, double *quats, int64_t n_quat_buf,
-                      const int32_t *pixel_index, int64_t *pixels, int64_t n_pix_buf,
-                      const int32_t *weight_index, double *weights, int64_t n_w_buf,
-                      const double *hwp, const tb_interval *intervals, int64_t n_view,
-                      uint8_t *hit_submaps, int64_t n_submap, int64_t n_pix_submap, int64_t nside,
-                      int nest, const double *epsilon, const double *gamma, const double *cal,
-                      int IAU, int64_t n_det, int64_t n_samp, int mem, void *stream) {
-    TB_API_BEGIN
-    tbr::Resolver R(mem, stream);
-    TB_REQUIRE(nside > 0 && (nside & (nside - 1)) == 0, "nside must be a power of two");
-    TB_REQUIRE(nside <= (1 << 24), "nside > 2^24 not supported");
+} // extern "C"
+
+namespace {
+
+// the body of tb_pointing_fused / tb_pointing_fused_wcs: `n_pix_map` is the number of pixels the
+// hit-submap mask must cover
+template <class PIX>
+void pointing_fused(tbr::Resolver &R, const typename PIX::Geom &geom, int64_t n_pix_map,
+                    const char *hsub_msg, const double *focalplane, const double *boresight,
+                    const uint8_t *shared_flags, uint8_t shared_flag_mask,
+                    const int32_t *quat_index, double *quats, int64_t n_quat_buf,
+                    const int32_t *pixel_index, int64_t *pixels, int64_t n_pix_buf,
+                    const int32_t *weight_index, double *weights, int64_t n_w_buf,
+                    const double *hwp, const tb_interval *intervals, int64_t n_view,
+                    uint8_t *hit_submaps, int64_t n_submap, int64_t n_pix_submap,
+                    const double *epsilon, const double *gamma, const double *cal, int IAU,
+                    int64_t n_det, int64_t n_samp) {
     Views V = make_views(R, intervals, n_view, n_samp);
     FusedOut o{};
     if (quats) {
@@ -777,8 +761,7 @@ int tb_pointing_fused(const double *focalplane, const double *boresight,
         o.pidx = R.small(pixel_index, n_det);
         o.pixels = R.out(pixels, n_pix_buf * n_samp);
         if (hit_submaps) {
-            TB_REQUIRE(n_pix_submap > 0 && n_submap * n_pix_submap >= 12 * nside * nside,
-                       "hit_submaps too small for nside");
+            TB_REQUIRE(n_pix_submap > 0 && n_submap * n_pix_submap >= n_pix_map, hsub_msg);
             o.hsub = R.small_inout(hit_submaps, n_submap);
         }
     }
@@ -795,22 +778,66 @@ int tb_pointing_fused(const double *focalplane, const double *boresight,
     const double *d_bore = R.in(boresight, 4 * n_samp);
     const uint8_t *d_fl = R.in(shared_flags, n_samp);
     const double *d_hwp = R.in(hwp, n_samp);
-    tbm::PixCtx ctx = tbm::make_pix_ctx(nside, g_guard_scale);
     double inv = 1.0 / (double)(n_pix_submap > 0 ? n_pix_submap : 1);
     double U_sign = IAU ? -1.0 : 1.0;
     int64_t nb = n_blocks(V, n_det);
-#define TB_FUSED(NEST, HWP)                                                                    \
-    {                                                                                          \
-        auto kfn = k_pointing_fused<NEST, HWP>;                                                \
-        TB_LAUNCH(kfn, nb, R, V, n_det, n_samp, ctx, d_fp, d_bore, d_fl, shared_flag_mask, o,  \
-                  d_hwp, d_eps, d_gam, d_cal, U_sign, inv);                                    \
-    }
-    if (nest) {
-        if (d_hwp) TB_FUSED(true, true) else TB_FUSED(true, false)
+    if (d_hwp) {
+        auto kfn = k_pointing_fused<PIX, true>;
+        TB_LAUNCH(kfn, nb, R, V, n_det, n_samp, geom, d_fp, d_bore, d_fl, shared_flag_mask, o,
+                  d_hwp, d_eps, d_gam, d_cal, U_sign, inv);
     } else {
-        if (d_hwp) TB_FUSED(false, true) else TB_FUSED(false, false)
+        auto kfn = k_pointing_fused<PIX, false>;
+        TB_LAUNCH(kfn, nb, R, V, n_det, n_samp, geom, d_fp, d_bore, d_fl, shared_flag_mask, o,
+                  d_hwp, d_eps, d_gam, d_cal, U_sign, inv);
     }
-#undef TB_FUSED
+}
+
+} // namespace
+
+extern "C" {
+
+int tb_pointing_fused(const double *focalplane, const double *boresight,
+                      const uint8_t *shared_flags, uint8_t shared_flag_mask,
+                      const int32_t *quat_index, double *quats, int64_t n_quat_buf,
+                      const int32_t *pixel_index, int64_t *pixels, int64_t n_pix_buf,
+                      const int32_t *weight_index, double *weights, int64_t n_w_buf,
+                      const double *hwp, const tb_interval *intervals, int64_t n_view,
+                      uint8_t *hit_submaps, int64_t n_submap, int64_t n_pix_submap, int64_t nside,
+                      int nest, const double *epsilon, const double *gamma, const double *cal,
+                      int IAU, int64_t n_det, int64_t n_samp, int mem, void *stream) {
+    TB_API_BEGIN
+    tbr::Resolver R(mem, stream);
+    TB_REQUIRE(nside > 0 && (nside & (nside - 1)) == 0, "nside must be a power of two");
+    TB_REQUIRE(nside <= (1 << 24), "nside > 2^24 not supported");
+    tbm::PixCtx ctx = tbm::make_pix_ctx(nside, g_guard_scale);
+    auto fused = nest ? pointing_fused<tbp::PixHealpix<true>>
+                      : pointing_fused<tbp::PixHealpix<false>>;
+    fused(R, ctx, 12 * nside * nside, "hit_submaps too small for nside", focalplane, boresight,
+          shared_flags, shared_flag_mask, quat_index, quats, n_quat_buf, pixel_index, pixels,
+          n_pix_buf, weight_index, weights, n_w_buf, hwp, intervals, n_view, hit_submaps,
+          n_submap, n_pix_submap, epsilon, gamma, cal, IAU, n_det, n_samp);
+    R.finish();
+    TB_API_END
+}
+
+int tb_pointing_fused_wcs(const double *focalplane, const double *boresight,
+                          const uint8_t *shared_flags, uint8_t shared_flag_mask,
+                          const int32_t *quat_index, double *quats, int64_t n_quat_buf,
+                          const int32_t *pixel_index, int64_t *pixels, int64_t n_pix_buf,
+                          const int32_t *weight_index, double *weights, int64_t n_w_buf,
+                          const double *hwp, const tb_interval *intervals, int64_t n_view,
+                          uint8_t *hit_submaps, int64_t n_submap, int64_t n_pix_submap,
+                          const tb_wcs_desc *wcs, const double *epsilon, const double *gamma,
+                          const double *cal, int IAU, int64_t n_det, int64_t n_samp, int mem,
+                          void *stream) {
+    TB_API_BEGIN
+    tbr::Resolver R(mem, stream);
+    tbw::Wcs w = tbp::wcs_from_desc(wcs);
+    pointing_fused<tbp::PixWcs>(R, w, w.n_pix, "hit_submaps too small for the projection",
+                                focalplane, boresight, shared_flags, shared_flag_mask, quat_index,
+                                quats, n_quat_buf, pixel_index, pixels, n_pix_buf, weight_index,
+                                weights, n_w_buf, hwp, intervals, n_view, hit_submaps, n_submap,
+                                n_pix_submap, epsilon, gamma, cal, IAU, n_det, n_samp);
     R.finish();
     TB_API_END
 }

@@ -10,7 +10,10 @@
 //   pass 2 (k_project)  out[amp(s)] += w_det * ((F a)[s] - sum_k weights[s,k] * map[pix,k])
 // With stored pointing a pass streams 33 B per det-sample (pixel 8 + weights 24 + flag 1); with
 // REGEN the pointing is recomputed from the boresight in registers and only the flag byte is read.
+#include <type_traits>
+
 #include "tb_device.cuh"
+#include "tb_pixelise.cuh"
 #include "tb_runtime.cuh"
 
 using namespace tbd;
@@ -27,7 +30,8 @@ struct ObsDev {
     const double *fp, *cal, *eta, *gamma, *det_scale;
     double inv_step, inv_nps;
     int64_t n_pix_submap;
-    tbm::PixCtx ctx;
+    tbm::PixCtx ctx; // HEALPix observations
+    tbw::Wcs wcs;    // WCS observations
     double U_sign;
     const double *boresight;
     const uint8_t *shared_flags;
@@ -56,8 +60,9 @@ __device__ unsigned long long g_exact_count_solver = 0ull;
 #endif
 constexpr int kBinRunCap = TB_BIN_RUN_CAP; // see find_runs<CAP>
 
-// pixel + weights of one sample, either streamed from HBM or regenerated from the boresight
-template <bool REGEN, bool NEST>
+// pixel + weights of one sample, either streamed from HBM or regenerated from the boresight with
+// the pixelisation policy PIX (tb_pixelise.cuh: the device function tb_pointing_fused[_wcs] runs)
+template <bool REGEN, class PIX>
 __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_t s, bool need,
                                                 int64_t &pix, double &w0, double &w1, double &w2,
                                                 int &n_exact) {
@@ -75,11 +80,11 @@ __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_
         if (bad || !need) return;
         tbm::Quat f = ld_quat(o.fp + 4 * det);
         tbm::Quat q = tbm::qmul(ld_quat(o.boresight + 4 * s), f);
-        double dx, dy, dz;
-        tbm::rot_zaxis(q, dx, dy, dz);
-        int ex = 0;
-        pix = tbm::vec2pix<NEST>(o.ctx, dx, dy, dz, &ex);
-        n_exact += ex;
+        if constexpr (std::is_same_v<typename PIX::Geom, tbw::Wcs>) {
+            pix = PIX::pixel(o.wcs, q, n_exact);
+        } else {
+            pix = PIX::pixel(o.ctx, q, n_exact);
+        }
         double cal = __ldg(o.cal + det), eta = __ldg(o.eta + det);
         if (o.hwp) {
             tbm::stokes_iqu<true>(q, cal, eta, o.U_sign, __ldg(o.gamma + det), __ldg(o.hwp + s), w0,
@@ -114,7 +119,7 @@ __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_
 #ifndef TB_REGEN_CTAS
 #define TB_REGEN_CTAS 4
 #endif
-template <bool REGEN, bool NEST, bool FROM_SIGNAL>
+template <bool REGEN, class PIX, bool FROM_SIGNAL>
 __global__ void __launch_bounds__(kThreads, REGEN ? TB_REGEN_CTAS : 6)
 k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ aflags,
       const double *__restrict__ signal, double *__restrict__ zmap) {
@@ -136,7 +141,7 @@ k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ afl
             }
             int64_t pix;
             double w0, w1, w2;
-            sample_pointing<REGEN, NEST>(o, det, s, ok, pix, w0, w1, w2, n_exact);
+            sample_pointing<REGEN, PIX>(o, det, s, ok, pix, w0, w1, w2, n_exact);
             if (ok && pix >= 0) {
                 int64_t gsm = fast_div(pix, o.inv_nps);
                 key = __ldg(o.g2l + gsm) * o.n_pix_submap + (pix - gsm * o.n_pix_submap);
@@ -161,7 +166,7 @@ k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ afl
 }
 
 // ---- pass 2: (template - scanned map) -> noise weight -> template projection ------------------
-template <bool REGEN, bool NEST, bool FROM_SIGNAL>
+template <bool REGEN, class PIX, bool FROM_SIGNAL>
 __global__ void __launch_bounds__(kThreads, REGEN ? TB_REGEN_CTAS : 6)
 k_project(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ aflags,
           const double *__restrict__ signal, const double *__restrict__ binned,
@@ -189,7 +194,7 @@ k_project(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__
             }
             int64_t pix;
             double w0, w1, w2;
-            sample_pointing<REGEN, NEST>(o, det, s, need, pix, w0, w1, w2, n_exact);
+            sample_pointing<REGEN, PIX>(o, det, s, need, pix, w0, w1, w2, n_exact);
             if (need) {
                 if (pix >= 0) {
                     int64_t gsm = fast_div(pix, o.inv_nps);
@@ -1389,7 +1394,13 @@ ObsDev make_dev(const tb_obs *obs, int regen) {
     o.inv_step = 1.0 / (double)d.step_length;
     o.inv_nps = 1.0 / (double)d.n_pix_submap;
     o.n_pix_submap = d.n_pix_submap;
-    o.ctx = tbm::make_pix_ctx(d.nside, 1.0);
+    if (obs->is_wcs) {
+        o.ctx = tbm::PixCtx{};
+        o.wcs = obs->wcs;
+    } else {
+        o.ctx = tbm::make_pix_ctx(d.nside, 1.0);
+        o.wcs = tbw::Wcs{};
+    }
     o.U_sign = d.IAU ? -1.0 : 1.0;
     o.boresight = d.boresight;
     o.shared_flags = d.shared_flags;
@@ -1565,13 +1576,16 @@ void launch_bin(const tb_obs *obs, const double *amps, const uint8_t *aflags, co
     } else if (!regen && !FROM_SIGNAL && tma_ok(o)) {
         launch_tma<false>(o, amps, aflags, nullptr, zmap, stream);
     } else if (!regen) {
-        auto k = k_bin<false, true, FROM_SIGNAL>;
+        auto k = k_bin<false, tbp::PixHealpix<true>, FROM_SIGNAL>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+    } else if (obs->is_wcs) {
+        auto k = k_bin<true, tbp::PixWcs, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
     } else if (obs->d.nest) {
-        auto k = k_bin<true, true, FROM_SIGNAL>;
+        auto k = k_bin<true, tbp::PixHealpix<true>, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
     } else {
-        auto k = k_bin<true, false, FROM_SIGNAL>;
+        auto k = k_bin<true, tbp::PixHealpix<false>, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
     }
 }
@@ -1607,13 +1621,16 @@ void launch_project(const tb_obs *obs, const double *amps, const uint8_t *aflags
     } else if (!regen && !FROM_SIGNAL && tma_ok(o)) {
         launch_tma<true>(o, amps, aflags, binned, out, stream);
     } else if (!regen) {
-        auto k = k_project<false, true, FROM_SIGNAL>;
+        auto k = k_project<false, tbp::PixHealpix<true>, FROM_SIGNAL>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+    } else if (obs->is_wcs) {
+        auto k = k_project<true, tbp::PixWcs, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
     } else if (obs->d.nest) {
-        auto k = k_project<true, true, FROM_SIGNAL>;
+        auto k = k_project<true, tbp::PixHealpix<true>, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
     } else {
-        auto k = k_project<true, false, FROM_SIGNAL>;
+        auto k = k_project<true, tbp::PixHealpix<false>, FROM_SIGNAL>;
         TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
     }
 }
@@ -1750,19 +1767,33 @@ void tb_launch_prescale(const tb_obs *obs, const double *amps, const uint8_t *af
 
 extern "C" {
 
-tb_obs *tb_obs_create(const tb_obs_desc *desc) {
+} // extern "C"
+
+namespace {
+
+// the body of tb_obs_create / tb_obs_create_wcs; `wcs` NULL: a HEALPix observation
+tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
     try {
         tbr::require_device();
         TB_REQUIRE(desc != nullptr, "NULL descriptor");
         const tb_obs_desc &d = *desc;
         TB_REQUIRE(d.n_det > 0 && d.n_samp > 0 && d.n_view >= 0, "bad observation shape");
         TB_REQUIRE(d.step_length > 0, "step_length must be positive");
-        TB_REQUIRE(d.nside > 0 && (d.nside & (d.nside - 1)) == 0 && d.nside <= (1 << 24),
-                   "nside must be a power of two <= 2^24");
+        tbw::Wcs w{};
+        if (wcs) {
+            w = tbp::wcs_from_desc(wcs);
+            TB_REQUIRE(d.n_pix_submap > 0 && d.n_submap * d.n_pix_submap >= w.n_pix,
+                       "the submaps do not cover the projection");
+        } else {
+            TB_REQUIRE(d.nside > 0 && (d.nside & (d.nside - 1)) == 0 && d.nside <= (1 << 24),
+                       "nside must be a power of two <= 2^24");
+        }
         TB_REQUIRE(d.global2local && d.det_scale && d.amp_offsets && d.n_amp_views && d.intervals,
                    "missing descriptor arrays");
         tb_obs *o = new tb_obs();
         o->d = d;
+        o->is_wcs = wcs != nullptr;
+        o->wcs = w;
         // pack: int64 [first(nv), prefix(nv+1), amp_view_off(nv), amp_offsets(nd), g2l(ns)]
         //       double [fp(4nd), cal, eta, gamma, det_scale]
         int64_t nv = d.n_view, nd = d.n_det, ns = d.n_submap;
@@ -1844,6 +1875,20 @@ tb_obs *tb_obs_create(const tb_obs_desc *desc) {
         tbr::set_error(e.code, e.msg);
         return nullptr;
     }
+}
+
+} // namespace
+
+extern "C" {
+
+tb_obs *tb_obs_create(const tb_obs_desc *desc) { return obs_create(desc, nullptr); }
+
+tb_obs *tb_obs_create_wcs(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
+    if (wcs == nullptr) {
+        tbr::set_error(TB_ERR_ARG, "NULL projection");
+        return nullptr;
+    }
+    return obs_create(desc, wcs);
 }
 
 void tb_obs_destroy(tb_obs *obs) {

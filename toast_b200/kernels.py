@@ -210,6 +210,42 @@ def pointing_fused(focalplane, boresight, shared_flags, shared_flag_mask, quat_i
         L.mem_of(big, use_accel), _stream(stream)))
 
 
+def pointing_fused_wcs(wcs, focalplane, boresight, shared_flags, shared_flag_mask, quat_index,
+                       quats, pixel_index, pixels, weight_index, weights, hwp, intervals,
+                       hit_submaps, n_pix_submap, epsilon, gamma, cal, IAU, use_accel=False,
+                       stream=None):
+    """``pointing_fused`` onto a flat projection: ``wcs`` is a ``toast_b200.wcs.FlatWCS`` (or
+    anything with a ``.desc()`` returning a tb_wcs_desc), as for ``pixels_wcs``."""
+    import ctypes as ct
+
+    _require(boresight, "boresight", "float64", 2)
+    n_samp = _shape(boresight)[0]
+    focalplane = L.host(focalplane, np.float64)
+    n_det = focalplane.shape[0]
+    iv = _intervals(intervals)
+    fl = _optional(shared_flags, n_samp)
+    h = _optional(hwp, n_samp)
+    qi = L.host(quat_index, np.int32) if quats is not None else None
+    pi = L.host(pixel_index, np.int32) if pixels is not None else None
+    wi = L.host(weight_index, np.int32) if weights is not None else None
+    eps = L.host(epsilon, np.float64)
+    gam = L.host(gamma, np.float64)
+    c = L.host(cal, np.float64)
+    if hit_submaps is not None and (L._is_tensor(hit_submaps) or hit_submaps.dtype != np.uint8):
+        raise RuntimeError("Object hit_submaps must be a host uint8 array")
+    d = wcs.desc()
+    big = pixels if pixels is not None else (weights if weights is not None else quats)
+    L.check(L.load().tb_pointing_fused_wcs(
+        L.ptr(focalplane), L.ptr(boresight), L.ptr(fl), shared_flag_mask,
+        L.ptr(qi), L.ptr(quats), _shape(quats)[0] if quats is not None else 0,
+        L.ptr(pi), L.ptr(pixels), _shape(pixels)[0] if pixels is not None else 0,
+        L.ptr(wi), L.ptr(weights), _shape(weights)[0] if weights is not None else 0,
+        L.ptr(h), L.ptr(iv), len(iv), L.ptr(hit_submaps),
+        len(hit_submaps) if hit_submaps is not None else 0, n_pix_submap, ct.byref(d),
+        L.ptr(eps), L.ptr(gam), L.ptr(c), 1 if IAU else 0, n_det, n_samp,
+        L.mem_of(big, use_accel), _stream(stream)))
+
+
 def noise_weight(det_data, data_index, intervals, detector_weights, use_accel=False,
                  stream=None):
     """ops_noise_weight.cpp:12-118."""

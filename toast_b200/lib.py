@@ -99,6 +99,9 @@ PROTOTYPES = {
     "tb_stokes_weights_I": (INT, [P, P, I64, P, I64, P, I64, I64, INT, P]),
     "tb_pointing_fused": (INT, [P, P, P, U8, P, P, I64, P, P, I64, P, P, I64, P, P, I64, P, I64,
                                 I64, I64, INT, P, P, P, INT, I64, I64, INT, P]),
+    "tb_pointing_fused_wcs": (INT, [P, P, P, U8, P, P, I64, P, P, I64, P, P, I64, P, P, I64, P,
+                                    I64, I64, ct.POINTER(tb_wcs_desc), P, P, P, INT, I64, I64,
+                                    INT, P]),
     "tb_noise_weight": (INT, [P, I64, P, P, I64, P, I64, I64, INT, P]),
     "tb_build_noise_weighted": (INT, [P, I64, P, I64, I64, I64, P, P, I64, P, P, I64, P, P, I64,
                                       P, P, I64, P, U8, P, I64, P, U8, I64, I64, INT, P]),
@@ -118,6 +121,7 @@ PROTOTYPES = {
                            P, I64, P, U8, I64, I64, INT, P]),
     "tb_cov_invert": (INT, [I64, I64, P, P, F64, INT, P]),
     "tb_obs_create": (P, [ct.POINTER(tb_obs_desc)]),
+    "tb_obs_create_wcs": (P, [ct.POINTER(tb_obs_desc), ct.POINTER(tb_wcs_desc)]),
     "tb_obs_destroy": (None, [P]),
     "tb_lhs_pass1": (INT, [P, P, P, P, INT, P]),
     "tb_lhs_pass2": (INT, [P, P, P, P, P, INT, P]),

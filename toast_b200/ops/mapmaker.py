@@ -15,6 +15,7 @@ from ..pixels import PixelData, PixelDistribution
 from ..templates.amplitudes import AmplitudesMap
 from ..templates.offset import Offset
 from .operator import Operator
+from .pixels_wcs import PixelsWCS
 
 
 def _identity_rows(dd, dets):
@@ -150,8 +151,11 @@ class TemplateMatrix(Operator):
 
 
 class MapMaker(Operator):
-    """Generalised destriper restricted to what the hot path covers: HEALPix pointing, I/Q/U
-    weights, a diagonal noise model and ONE ``templates.Offset`` template.
+    """Generalised destriper restricted to what the hot path covers: HEALPix
+    (``ops.PixelsHealpix``) or flat-sky WCS (``ops.PixelsWCS``) pointing, I/Q/U weights, a
+    diagonal noise model and ONE ``templates.Offset`` template.  With ``PixelsWCS`` the projection
+    is set up as that operator does (auto bounds from the boresights of every observation), and
+    the pixel distribution carries ``wcs`` / ``wcs_shape``.
 
     Products placed in ``data`` (names as in ``ops/mapmaker.py:382-651``):
     ``{name}_hits``, ``{name}_cov``, ``{name}_rcond``, ``{name}_binmap`` (raw binned map),
@@ -189,9 +193,15 @@ class MapMaker(Operator):
         if len(tmpls) != 1 or not isinstance(tmpls[0], Offset):
             raise NotImplementedError("MapMaker on the B200 path supports one Offset template")
         tmpl = tmpls[0]
+        is_wcs = isinstance(pixels, PixelsWCS)
         dp = pixels.detector_pointing
         view = pixels.view if pixels.view is not None else dp.view
-        pixels._geometry()
+        if is_wcs:
+            pixels._geometry(data)
+            pixelisation = dict(wcs=pixels.wcs)
+        else:
+            pixels._geometry()
+            pixelisation = dict(nside=pixels.nside, nest=pixels.nest)
         dev = torch.device(self.device)
         comm = data.comm
         # wall-clock per stage (device synchronised at every mark) when profile_stages is set
@@ -248,8 +258,7 @@ class MapMaker(Operator):
                 boresight=ob.shared[dp.boresight], intervals=iv,
                 det_scale=np.array([noise.detector_weight(x) for x in dets]),
                 step_length=tmpl._step_length(tmpl.step_time, tmpl._obs_rate[iob]),
-                nside=pixels.nside, nest=pixels.nest, n_pix_submap=pixels._n_pix_submap,
-                n_submap=pixels._n_submap,
+                n_pix_submap=pixels._n_pix_submap, n_submap=pixels._n_submap,
                 global2local=np.zeros(pixels._n_submap, dtype=np.int64),
                 epsilon=np.array([fp[x]["epsilon"] for x in dets]),
                 gamma=np.array([fp[x]["gamma"] for x in dets]),
@@ -259,7 +268,7 @@ class MapMaker(Operator):
                 hwp=ob.shared[weights.hwp_angle] if weights.hwp_angle is not None else None,
                 amp_offsets=np.array([tmpl._obs_amp_offset(x, iob) for x in dets],
                                      dtype=np.int64),
-                device=dev)
+                device=dev, **pixelisation)
             dobs.append(d)
             # the timestreams are not needed before the RHS: their upload (the largest transfer)
             # runs on its own stream, underneath the pointing expansion, the covariance and the
@@ -279,7 +288,11 @@ class MapMaker(Operator):
             comm.allreduce_(hits, op="max")
         local = np.flatnonzero(hits).astype(np.int64)
         dist = PixelDistribution(pixels._n_pix, pixels._n_submap, local, comm=comm.comm_world)
-        dist.nest = bool(pixels.nest)
+        if is_wcs:
+            dist.wcs = pixels.wcs
+            dist.wcs_shape = tuple(pixels.wcs_shape)
+        else:
+            dist.nest = bool(pixels.nest)
         data[binning.pixel_dist] = dist
         for d in dobs:
             d.set_global2local(dist.global_submap_to_local)

@@ -94,12 +94,17 @@ class PixelsWCS(Operator):
         if self.n_row < 1 or self.n_col < 1:
             raise RuntimeError(f"The WCS has non-positive dimensions: {self.wcs_shape}")
         self._n_pix = self.n_row * self.n_col
+        self._n_submap = self.submaps
         self._n_pix_submap = self._n_pix // self.submaps
         if self._n_pix_submap * self.submaps < self._n_pix:
             self._n_pix_submap += 1
         self._local_submaps = np.zeros(self.submaps, dtype=np.uint8)
 
-    def _exec(self, data, detectors=None, use_accel=False, **kwargs):
+    def _geometry(self, data):
+        """The projection of this operator for ``data``: with ``auto_bounds``, the bounds of the
+        boresights of every observation plus the field of view (pixels_wcs.py:436-489), then
+        ``set_wcs``.  Sets ``wcs``, ``wcs_shape`` and the pixel / submap counts; ops.MapMaker
+        calls it too."""
         if self.detector_pointing is None:
             raise RuntimeError("The detector_pointing trait must be set")
         for trait in ("fits_header", "center_offset"):
@@ -126,6 +131,10 @@ class PixelsWCS(Operator):
                 self.dimensions = ()
             self.auto_bounds = False
         self.set_wcs()
+
+    def _exec(self, data, detectors=None, use_accel=False, **kwargs):
+        self._geometry(data)
+        dp = self.detector_pointing
         view = self.view if self.view is not None else dp.view
         dp.apply(data, detectors=detectors, use_accel=use_accel)
         for ob in data.obs:

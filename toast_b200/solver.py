@@ -43,13 +43,20 @@ def _dev_tensor(a, device, dtype=None):
 class DeviceObservation:
     """One observation resident on the device, in the reference's buffer layouts
     (``detdata`` [n_det, n_samp, ...], ``shared`` [n_samp, ...]) plus the Offset amplitude
-    layout (``templates/offset/offset.py:245-253``: detector-major, ceil(len/step) per view)."""
+    layout (``templates/offset/offset.py:245-253``: detector-major, ceil(len/step) per view).
 
-    def __init__(self, *, focalplane, boresight, intervals, det_scale, step_length, nside, nest,
-                 n_pix_submap, n_submap, global2local, amp_offset=0, epsilon=None, gamma=None,
-                 cal=None, IAU=False, shared_flags=None, shared_flag_mask=0, solver_flags=None,
-                 solver_flag_mask=255, pixels=None, weights=None, hwp=None, amp_offsets=None,
-                 compact=True, device="cuda"):
+    The pixelisation is HEALPix (``nside`` / ``nest``) or a flat projection (``wcs``, a
+    ``toast_b200.wcs.FlatWCS`` with its shape set), one or the other."""
+
+    def __init__(self, *, focalplane, boresight, intervals, det_scale, step_length, n_pix_submap,
+                 n_submap, global2local, nside=None, nest=None, wcs=None, amp_offset=0,
+                 epsilon=None, gamma=None, cal=None, IAU=False, shared_flags=None,
+                 shared_flag_mask=0, solver_flags=None, solver_flag_mask=255, pixels=None,
+                 weights=None, hwp=None, amp_offsets=None, compact=True, device="cuda"):
+        if wcs is not None and (nside is not None or nest is not None):
+            raise ValueError("DeviceObservation takes either wcs or nside / nest, not both")
+        if wcs is None and (nside is None or nest is None):
+            raise ValueError("DeviceObservation needs nside and nest, or wcs")
         self.device = torch.device(device)
         self.lib = L.load()
         self.n_det = int(focalplane.shape[0])
@@ -61,7 +68,10 @@ class DeviceObservation:
         self.gamma = np.zeros(self.n_det) if gamma is None else np.ascontiguousarray(gamma)
         self.cal = np.ones(self.n_det) if cal is None else np.ascontiguousarray(cal)
         self.det_scale = np.ascontiguousarray(det_scale, dtype=np.float64)
-        self.nside, self.nest, self.IAU = int(nside), bool(nest), bool(IAU)
+        self.wcs = wcs
+        self.nside = None if wcs is not None else int(nside)
+        self.nest = None if wcs is not None else bool(nest)
+        self.IAU = bool(IAU)
         self.n_pix_submap, self.n_submap = int(n_pix_submap), int(n_submap)
         self.global2local = np.ascontiguousarray(global2local, dtype=np.int64)
         self.shared_flag_mask = int(shared_flag_mask)
@@ -96,8 +106,9 @@ class DeviceObservation:
 
     # -- pointing -----------------------------------------------------------------------------
     def expand_pointing(self, hit_submaps=None):
-        """PointingDetectorSimple -> PixelsHealpix -> StokesWeights in one fused kernel; fills
-        ``pixels`` / ``weights`` on the device and ORs the hit-submap mask (host uint8)."""
+        """PointingDetectorSimple -> PixelsHealpix (or PixelsWCS) -> StokesWeights in one fused
+        kernel; fills ``pixels`` / ``weights`` on the device and ORs the hit-submap mask (host
+        uint8)."""
         dev = self.device
         if self.pixels is None:
             self.pixels = torch.zeros((self.n_det, self.n_samp), dtype=torch.int64, device=dev)
@@ -105,10 +116,17 @@ class DeviceObservation:
             self.weights = torch.zeros((self.n_det, self.n_samp, 3), dtype=torch.float64,
                                        device=dev)
         idx = np.arange(self.n_det, dtype=np.int32)
-        K.pointing_fused(self.focalplane, self.boresight, self.shared_flags,
-                         self.shared_flag_mask, None, None, idx, self.pixels, idx, self.weights,
-                         self.hwp, self.intervals, hit_submaps, self.n_pix_submap, self.nside,
-                         self.nest, self.epsilon, self.gamma, self.cal, self.IAU)
+        if self.wcs is not None:
+            K.pointing_fused_wcs(self.wcs, self.focalplane, self.boresight, self.shared_flags,
+                                 self.shared_flag_mask, None, None, idx, self.pixels, idx,
+                                 self.weights, self.hwp, self.intervals, hit_submaps,
+                                 self.n_pix_submap, self.epsilon, self.gamma, self.cal, self.IAU)
+        else:
+            K.pointing_fused(self.focalplane, self.boresight, self.shared_flags,
+                             self.shared_flag_mask, None, None, idx, self.pixels, idx,
+                             self.weights, self.hwp, self.intervals, hit_submaps,
+                             self.n_pix_submap, self.nside, self.nest, self.epsilon, self.gamma,
+                             self.cal, self.IAU)
         self._handle = None
 
     def set_global2local(self, g2l):
@@ -137,8 +155,9 @@ class DeviceObservation:
         d.amp_offsets = self.amp_offsets.ctypes.data
         d.n_amp_views = self.n_amp_views.ctypes.data
         d.step_length = self.step_length
-        d.nside, d.n_pix_submap, d.n_submap = self.nside, self.n_pix_submap, self.n_submap
-        d.nest, d.IAU = int(self.nest), int(self.IAU)
+        d.nside = 0 if self.wcs is not None else self.nside
+        d.n_pix_submap, d.n_submap = self.n_pix_submap, self.n_submap
+        d.nest, d.IAU = int(bool(self.nest)), int(self.IAU)
         d.global2local = self.global2local.ctypes.data
         d.boresight = L.ptr(self.boresight)
         d.shared_flags = L.ptr(self.shared_flags)
@@ -148,7 +167,11 @@ class DeviceObservation:
         d.pixels = L.ptr(self.pixels)
         d.weights = L.ptr(self.weights)
         d.hwp = L.ptr(self.hwp)
-        h = self.lib.tb_obs_create(ct.byref(d))
+        if self.wcs is not None:
+            self._wcs_desc = self.wcs.desc()
+            h = self.lib.tb_obs_create_wcs(ct.byref(d), ct.byref(self._wcs_desc))
+        else:
+            h = self.lib.tb_obs_create(ct.byref(d))
         if not h:
             raise RuntimeError(L.last_error())
         self._handle = _ObsHandle(self.lib, h)
