@@ -71,6 +71,17 @@ def test_runtime_queries_work_without_gpu():
     assert lib.tb_accel_enabled() in (0, 1)
 
 
+def test_removed_lhs_options_are_unknown():
+    """The LHS paths that only an option could reach are gone, and so are their switches."""
+    lib = tbl.load()
+    for name in (b"tma", b"compact", b"sorted", b"sorted2"):
+        assert lib.tb_get_option(name) == -1, name
+        assert lib.tb_set_option(name, 1) == tbl.TB_ERR_ARG, name
+        assert "unknown option" in tbl.last_error()
+    for name in (b"blocked", b"crossings", b"pair", b"pairw"):
+        assert lib.tb_get_option(name) in (0, 1), name
+
+
 def test_no_cpu_fallback():
     """Without a device every compute entry point must fail loudly, not compute on the CPU."""
     import numpy as np

@@ -383,22 +383,16 @@ def test_pixel_chunked_passes(dyadic):
         L.check(lib.tb_obs_set_pixel_chunks(d.h, 1, L.ptr(whole)))
 
 
-# the kernel variants of test_gpu_solver.py::test_lhs_kernel_variants_agree
-VARIANTS = (("sorted2", dict(blocked=0, sorted=1, sorted2=1, crossings=1, pair=1, pairw=1,
-                             compact=1, tma=0)),
-            ("sorted", dict(sorted=1, sorted2=0, crossings=1, pair=1, pairw=1, compact=1, tma=0)),
-            ("crossings", dict(sorted=0, crossings=1, pair=1, pairw=1, compact=1, tma=0)),
-            ("pairw", dict(crossings=0, pair=1, pairw=1, compact=1, tma=0)),
-            ("pair", dict(crossings=0, pair=1, pairw=0, compact=1, tma=0)),
-            ("compact", dict(crossings=0, pair=0, compact=1, tma=0)),
-            ("tma", dict(crossings=0, pair=0, compact=0, tma=1)),
-            ("general", dict(crossings=0, pair=0, compact=0, tma=0)))
-DEFAULT_OPTIONS = dict(blocked=1, sorted=1, sorted2=1, crossings=1, pair=1, pairw=1, compact=1,
-                       tma=0)
+# the kernel variants of test_gpu_solver.py::test_lhs_path_variants_agree
+VARIANTS = (("crossings", dict(blocked=0, crossings=1, pair=1, pairw=1)),
+            ("pairw", dict(blocked=0, crossings=0, pair=1, pairw=1)),
+            ("pair", dict(blocked=0, crossings=0, pair=1, pairw=0)),
+            ("general", dict(blocked=0, crossings=0, pair=0)))
+DEFAULT_OPTIONS = dict(blocked=1, crossings=1, pair=1, pairw=1)
 
 
 @pytest.mark.gpu
-def test_kernel_variants_are_exact(dyadic):
+def test_lhs_path_variants_are_exact(dyadic):
     """Every other LHS kernel, and the regenerated-pointing form, on the same inputs."""
     lib = L.load()
     d = dyadic

@@ -16,8 +16,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("TB_LIB_PATH", os.path.join(HERE, "libtoastb200.so"))
 SOURCES = ["tb_runtime.cu", "tb_ops.cu", "tb_solver.cu", "tb_blocked.cu", "tb_peer.cu",
            "tb_sort.cu", "tb_prior.cu"]
-HEADERS = ["tb_math.cuh", "tb_device.cuh", "tb_runtime.cuh", "tb_prior.cuh", "tb_obs.cuh", "tb_tma.cuh",
-           "tb_wcs.cuh", "tb_pixelise.cuh",
+HEADERS = ["tb_math.cuh", "tb_device.cuh", "tb_runtime.cuh", "tb_prior.cuh", "tb_obs.cuh", "tb_wcs.cuh",
+           "tb_pixelise.cuh",
            "../../include/toast_b200.h"]
 
 NVCC_FLAGS = [

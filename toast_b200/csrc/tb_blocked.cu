@@ -589,7 +589,7 @@ void tb_build_blocked(tb_obs *obs, cudaStream_t st) {
     tb_free_blocked(obs);
     const int64_t n_rec = obs->n_xrec, nad = obs->n_amp_det, n_det = obs->d.n_det;
     const int64_t n_pix = obs->n_local_pix;
-    if (obs->xrec == nullptr || obs->stable == nullptr || obs->dscaled == nullptr) return;
+    if (obs->xrec == nullptr || obs->stable == nullptr) return;
     if (n_rec <= 0 || n_rec >= (1LL << 29) || n_det * nad >= 2147483647LL || n_pix <= 0 ||
         n_pix >= (1LL << 31) - kBxPix || obs->n_xrows > (1LL << kBxRowBits))
         return; // (the records carry their row in kBxRowBits bits)

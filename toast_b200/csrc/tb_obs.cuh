@@ -1,6 +1,6 @@
 // tb_obs.cuh -- the native observation handle shared by the solver translation units
-// (tb_solver.cu: per-sample, crossing-list and pixel-sorted passes; tb_blocked.cu: the
-// block-ordered crossing list with shared-memory map tiles).
+// (tb_solver.cu: per-sample and crossing-list passes; tb_blocked.cu: the block-ordered crossing
+// list with shared-memory map tiles).
 #pragma once
 
 #include <vector>
@@ -27,9 +27,6 @@ struct tb_obs {
     int is_wcs = 0; // pixels of a flat projection (tb_obs_create_wcs): regenerated with `wcs`
     tbw::Wcs wcs{};
     int64_t n_amp_det = 0;
-    // per-interval tiles for the TMA-staged passes: [n_tiles] x {s0, off, cnt, view}
-    int64_t *tiles = nullptr;
-    int64_t n_tiles = 0;
     // compact solver pointing (tb_obs_pack_pointing): local pixel (int32, <0 = nothing to do)
     // and the two sample-dependent weights (Q, U) as one 16-byte record
     int32_t *lpix = nullptr;
@@ -45,16 +42,7 @@ struct tb_obs {
     int4 *xblocks = nullptr;    // [n_xblocks] {row, first record, end record, 0}
     int64_t n_xrec = 0, n_xblocks = 0, n_xrows = 0;
     int x_paired = 0;           // rows are detector pairs (weights shared through pair_rot)
-    // pixel-sorted copy of the crossing list for pass 1 (see k_bin_xs)
-    int4 *srec = nullptr;       // [n_srec] {local pixel, scaled-amplitude index, n0|n1<<8|row<<16, 0}
-    double2 *squ = nullptr;     // [n_srec]
     double4 *stable = nullptr;  // [n_xrows] {cal0, cal1, A, B}
-    double *dscaled = nullptr;  // [n_det * n_amp_det] scratch: amplitude * det_scale, NaN-tagged if flagged
-    int64_t n_srec = 0;
-    int s_pass2_ok = 0;         // no unflagged off-map sample: pass 2 may run on the sorted list too
-    // pixel chunks of the sorted list (tb_obs_set_pixel_chunks): records of chunk c are
-    // [chunk_rec[c], chunk_rec[c + 1])
-    std::vector<int64_t> chunk_rec;
     // block-ordered crossing list (tb_blocked.cu): the time-ordered records stably sorted by
     // PIXEL BLOCK (kBxPix consecutive local pixels), i.e. in (block, row, time) order.  A CTA owns
     // one block at a time and keeps its 3 x kBxPix map values in shared memory.
@@ -74,16 +62,7 @@ struct tb_obs {
 
 
 // ---- shared between tb_solver.cu and tb_blocked.cu ---------------------------------------------
-// Flagged baselines are marked in the prescaled amplitude copy with a NaN of this bit pattern (an
-// arithmetic NaN never carries this payload, so a diverged solve still propagates its own NaNs).
-constexpr unsigned long long kAmpFlagBits = 0x7FF8000000B200B2ULL;
-__device__ __forceinline__ bool amp_is_flagged(double v) {
-    return (unsigned long long)__double_as_longlong(v) == kAmpFlagBits;
-}
-
-// dscaled <- amplitude x detector weight, flag folded in (k_amp_prescale, tb_solver.cu)
-void tb_launch_prescale(const tb_obs *obs, const double *amps, const uint8_t *aflags, void *stream);
-// per-row constants {cal0, cal1, A, B}, uniformity, and the prescale scratch (tb_solver.cu)
+// per-row constants {cal0, cal1, A, B} and their uniformity (tb_solver.cu)
 void tb_build_row_table(tb_obs *obs);
 // block-ordered crossing list (tb_blocked.cu); frees a previous one
 void tb_build_blocked(tb_obs *obs, cudaStream_t st);

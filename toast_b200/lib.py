@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("TB_LIB_PATH", os.path.join(HERE, "libtoastb200.so"))
 
 TB_MEM_HOST, TB_MEM_DEVICE, TB_MEM_TABLE = 0, 1, 2
-TB_ERR_NO_DEVICE = 2
+TB_ERR_NO_DEVICE, TB_ERR_ARG = 2, 3
 
 interval_dtype = np.dtype(
     {
@@ -127,9 +127,6 @@ PROTOTYPES = {
     "tb_lhs_pass2": (INT, [P, P, P, P, P, INT, P]),
     "tb_obs_sorted_passes": (INT, [P]),
     "tb_obs_set_pixel_chunks": (INT, [P, I64, P]),
-    "tb_lhs_pass1_chunk": (INT, [P, P, P, P, I64, P]),
-    "tb_lhs_pass2_chunk": (INT, [P, P, P, I64, P]),
-    "tb_lhs_pass2_cov": (INT, [P, P, P, P, P]),
     "tb_bx_block_pixels": (INT, []),
     "tb_obs_blocked": (INT, [P]),
     "tb_obs_blocked_stats": (INT, [P, P, P, P, P]),
@@ -184,7 +181,7 @@ def load():
         fn.restype = res
         fn.argtypes = args
     _lib = lib
-    # TB_OPTIONS="crossings=0,sorted=0": kernel-variant switches for A/B measurements
+    # TB_OPTIONS="blocked=0,crossings=0": kernel-variant switches for A/B measurements
     for item in os.environ.get("TB_OPTIONS", "").split(","):
         if "=" in item:
             k, v = item.split("=", 1)

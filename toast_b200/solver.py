@@ -437,7 +437,6 @@ class Destriper:
         # time it against the serial LHS on this node and keep the faster form), 0 (off) or K.
         # Measured on 2 GPUs: 1.46-1.54 ms against 1.69 ms per iteration with 4 chunks, slower
         # than serial with 8-16 (DESIGN.md section 5).
-        self.fuse_cov = _os.environ.get("TB_FUSE_COV", "0") == "1"
         # one observation on one GPU: pass 1 -> covariance -> pass 2 inside one kernel
         self.fuse_lhs = _os.environ.get("TB_FUSE_LHS", "1") != "0"
         self.pipeline = False
@@ -457,12 +456,6 @@ class Destriper:
                 self.pipeline = False
 
     # -- chunk pipeline -------------------------------------------------------------------------
-    def _sorted_passes(self):
-        """2 when BOTH passes of every observation run on the pixel-sorted crossing list."""
-        if self.regen:
-            return 0
-        return min(int(self.lib.tb_obs_sorted_passes(o.handle().h)) for o in self.obs)
-
     def _blocked(self):
         """True when the passes of every observation run on the block-ordered crossing list
         (shared-memory map tiles, tb_blocked.cu)."""
@@ -471,16 +464,16 @@ class Destriper:
         return all(bool(self.lib.tb_obs_blocked(o.handle().h)) for o in self.obs)
 
     def _setup_pipeline(self, n_chunks):
-        """Multi-GPU with both passes in pixel (block) order: cut the local map into pixel chunks
-        so that pass 1 of chunk c+1 and pass 2 of chunk c-1 overlap the NVLink reduction of chunk
-        c (the reduction runs on its own high-priority stream)."""
+        """Multi-GPU with both passes on the block-ordered crossing list: cut the local map into
+        pixel chunks so that pass 1 of chunk c+1 and pass 2 of chunk c-1 overlap the NVLink
+        reduction of chunk c (the reduction runs on its own high-priority stream)."""
         import os as _os
         self.blocked = self._blocked()
-        if self.peer is None or n_chunks < 2 or not (self.blocked or self._sorted_passes() == 2):
+        if self.peer is None or n_chunks < 2 or not self.blocked:
             return
         bounds = pipeline_chunk_bounds(
             self.n_local_submap * self.n_pix_submap, self.world, n_chunks,
-            align=int(self.lib.tb_bx_block_pixels()) if self.blocked else 1)
+            align=int(self.lib.tb_bx_block_pixels()))
         if bounds is None:
             return
         n_chunks = len(bounds) - 1
@@ -628,20 +621,14 @@ class Destriper:
             e1.record(stream)
             timeline.append((label, e0, e1))
 
-        blocked = getattr(self, "blocked", False)
         # (the block-ordered pass 1 writes every block of the map: no zero-fill)
-        timed("zero", main, lambda: (None if blocked else self.zmap.zero_(), amps_out.zero_()))
+        timed("zero", main, lambda: amps_out.zero_())
         for c in range(self.n_chunks):
             def p1(c=c):
                 for k, o in enumerate(self.obs):
-                    if blocked:
-                        L.check(self.lib.tb_bx_pass1(o.handle().h, L.ptr(amps_in),
-                                                     L.ptr(self.amp_flags), L.ptr(self.zmap),
-                                                     1 if k > 0 else 0, c, ms))
-                    else:
-                        L.check(self.lib.tb_lhs_pass1_chunk(o.handle().h, L.ptr(amps_in),
-                                                            L.ptr(self.amp_flags),
-                                                            L.ptr(self.zmap), c, ms))
+                    L.check(self.lib.tb_bx_pass1(o.handle().h, L.ptr(amps_in),
+                                                 L.ptr(self.amp_flags), L.ptr(self.zmap),
+                                                 1 if k > 0 else 0, c, ms))
             timed(f"pass1[{c}]", main, p1)
             self.ev_binned[c].record(main)
             self.comm_stream.wait_event(self.ev_binned[c])
@@ -655,12 +642,8 @@ class Destriper:
 
             def p2(c=c):
                 for o in self.obs:
-                    if blocked:
-                        L.check(self.lib.tb_bx_pass2(o.handle().h, L.ptr(self.zmap),
-                                                     L.ptr(amps_out), c, ms))
-                    else:
-                        L.check(self.lib.tb_lhs_pass2_chunk(o.handle().h, L.ptr(self.zmap),
-                                                            L.ptr(amps_out), c, ms))
+                    L.check(self.lib.tb_bx_pass2(o.handle().h, L.ptr(self.zmap), L.ptr(amps_out),
+                                                 c, ms))
             timed(f"pass2[{c}]", main, p2)
         return amps_out
 
@@ -689,15 +672,6 @@ class Destriper:
         L.check(self.lib.tb_cov_apply_diag(self.n_local_submap, self.n_pix_submap, 3,
                                            L.ptr(self.cov), L.ptr(self.zmap), L.TB_MEM_DEVICE,
                                            self._st()))
-
-    def bin_amplitudes(self, amps):
-        """binned = cov * allreduce(P^T N^-1 F a)   (BinMap with pre_process=TemplateMatrix)."""
-        self.zmap.zero_()
-        for o in self.obs:
-            L.check(self.lib.tb_lhs_pass1(o.handle().h, L.ptr(amps), L.ptr(self.amp_flags),
-                                          L.ptr(self.zmap), self.regen, self._st()))
-        self.reduce_and_apply_cov()
-        return self.zmap
 
     def bin_amplitudes_raw(self, amps):
         """This rank's raw noise-weighted map P^T N^-1 F a -- pass 1 only, no reduction, no
@@ -741,28 +715,14 @@ class Destriper:
                                           L.ptr(self.zmap), self.regen, self._st()))
         if ev:
             ev[1].record()
-        reuse = self._sorted_passes() == 2
-        if self.fuse_cov and reuse and self.world == 1 and len(self.obs) == 1:
-            # TB_FUSE_COV=1 (pixel-sorted path, option blocked=0): the covariance product is
-            # formed inside pass 2, the stand-alone covariance pass disappears
-            amps_out.zero_()
-            if ev:
-                ev[2].record()
-            L.check(self.lib.tb_lhs_pass2_cov(self.obs[0].handle().h, L.ptr(self.zmap),
-                                              L.ptr(self.cov), L.ptr(amps_out), self._st()))
-            if ev:
-                ev[3].record()
-                timers.append(ev)
-            return self._add_prior(amps_in, amps_out)
         self.reduce_and_apply_cov()
         amps_out.zero_()
         if ev:
             ev[2].record()
-        # both passes pixel-sorted: pass 2 reuses the prescaled amplitudes of pass 1
         for o in self.obs:
-            L.check(self.lib.tb_lhs_pass2(o.handle().h, None if reuse else L.ptr(amps_in),
-                                          L.ptr(self.amp_flags), L.ptr(self.zmap),
-                                          L.ptr(amps_out), self.regen, self._st()))
+            L.check(self.lib.tb_lhs_pass2(o.handle().h, L.ptr(amps_in), L.ptr(self.amp_flags),
+                                          L.ptr(self.zmap), L.ptr(amps_out), self.regen,
+                                          self._st()))
         if ev:
             ev[3].record()
             timers.append(ev)
