@@ -324,6 +324,16 @@ tb_obs *tb_obs_create(const tb_obs_desc *desc);
  * regenerated-pointing passes (regen != 0), which then compute the pixels tb_pointing_fused_wcs
  * stores.  Every other pass works on local pixel numbers and is the same for both kinds. */
 tb_obs *tb_obs_create_wcs(const tb_obs_desc *desc, const tb_wcs_desc *wcs);
+/* An INTENSITY observation (StokesWeights mode="I"): one Stokes value per pixel.  desc.weights
+ * points to [n_det, n_samp] (the I weights, equal to cal[det]); epsilon and gamma are ignored.
+ * `wcs` NULL: HEALPix pixels (nside / nest), otherwise as tb_obs_create_wcs.
+ * Every entry point below that takes a tb_obs accepts both kinds and sizes the map by the
+ * observation's nnz (tb_obs_nnz: 3 for tb_obs_create / tb_obs_create_wcs, 1 here): zmap / binned
+ * maps are [n_local_pix, nnz], covariances [n_local_pix, nnz (nnz + 1) / 2].  For an intensity
+ * observation tb_lhs_pass1 / tb_lhs_pass2 run the per-sample kernels (the "crossings", "pair" and
+ * "pairw" paths are IQU-only), and its crossing list keeps no (sum Q, sum U). */
+tb_obs *tb_obs_create_intensity(const tb_obs_desc *desc, const tb_wcs_desc *wcs /* NULL: HEALPix */);
+int tb_obs_nnz(const tb_obs *obs);
 void tb_obs_destroy(tb_obs *obs);
 
 int tb_lhs_pass1(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_flags,
@@ -354,7 +364,7 @@ int tb_obs_set_pixel_chunks(tb_obs *obs, int64_t n_chunks, const int64_t *pixel_
  *                (whole map or one pixel chunk) and ADDS to amplitudes_out.
  *   tb_bx_fused  one observation on one GPU: pass 1 -> covariance_apply (toast_map_cov.cpp:471-528)
  *                -> pass 2 inside one kernel, the map never leaves the SM.  zmap_scratch
- *                ([n_local_pix, 3]) is only touched for blocks that had to be cut into several
+ *                ([n_local_pix, nnz]) is only touched for blocks that had to be cut into several
  *                work units (high-contention maps).  ADDS to amplitudes_out.  amplitudes ==
  *                NULL: the amplitudes of the preceding tb_bx_fused / tb_bx_pass1 call. */
 int tb_bx_block_pixels(void);
@@ -475,7 +485,10 @@ int tb_obs_has_pair_weights(const tb_obs *obs);
 /* Crossing list built by tb_obs_pack_pointing: consecutive samples of a detector (pair) that share
  * the pixel and the baseline are collapsed into one 32-byte record {lp0, lp1, n, amp | sum Q,
  * sum U}; both LHS passes are linear in the weights, so they stream records instead of samples
- * (tb_solver.cu: k_lhs_x).  Built only when it is the smaller stream.  n_records = 0: not built. */
+ * (tb_solver.cu: k_lhs_x).  Built only when it is the smaller stream.  n_records = 0: not built.
+ * Intensity observations: 16-byte records {lp0, lp1, n, amp} (no weight sums), always built; their
+ * rows are detector pairs only when that gives the block-ordered list fewer entries (a record
+ * whose two detectors fall in different pixels takes two), and pairs need no weight relation. */
 int tb_obs_crossing_stats(const tb_obs *obs, int64_t *n_records, int64_t *n_rows, int *paired);
 
 /* Runtime options (A/B measurements, debugging; each LHS switch selects a path that is the only

@@ -33,6 +33,8 @@
 // On one GPU with one observation nothing has to leave the SM between the passes: the fused
 // kernel (k_bx<2>) accumulates the tile, applies the 3x3 pixel covariance in shared memory and
 // projects the same records (second read served by the L2) -- the map never touches HBM.
+// Intensity-only observations (tb_obs::nnz = 1) run the same kernels with NNZ = 1: records
+// without (sum Q, sum U), a tile of kBxPix doubles per warp and one tile update per record.
 #include <algorithm>
 
 #include "tb_obs.cuh"
@@ -99,6 +101,7 @@ k_bx_keys(const int4 *__restrict__ xrec, int64_t n_rec, int32_t n_blocks, int32_
     }
 }
 
+template <int NNZ> // 1: intensity records carry no (sum Q, sum U)
 __global__ void __launch_bounds__(kThreads)
 k_bx_gather(const int4 *__restrict__ xrec, const double2 *__restrict__ xqu,
             const int32_t *__restrict__ vals, int64_t n_sorted, int64_t n_amp_det, int row_in_rec,
@@ -116,7 +119,7 @@ k_bx_gather(const int4 *__restrict__ xrec, const double2 *__restrict__ xqu,
         brec[j] = make_int2((pix & (kBxPix - 1)) | (n0 << kBxShift) | (n1 << (kBxShift + 6)) |
                                 (row_in_rec ? (row << (kBxShift + 12)) : 0),
                             (int32_t)((int64_t)row * n_amp_det + r.w));
-        bqu[j] = xqu[i];
+        if constexpr (NNZ == 3) bqu[j] = xqu[i];
     }
 }
 
@@ -171,7 +174,7 @@ k_bx_prescale(int paired, int n_det, int64_t nad, const int64_t *__restrict__ am
 struct BxArgs {
     const int4 *units;        // {block, first record, end record, multi}
     const int2 *brec;
-    const double2 *bqu;
+    const double2 *bqu;       // NULL for intensity observations
     const double *ascaled;    // k_bx_prescale
     double *out;              // pass 2 / fused: amplitudes (REDs)
     const int64_t *amp_offsets;
@@ -181,7 +184,7 @@ struct BxArgs {
     double inv_nad;           // 1 / n_amp_det
     int64_t n_pix;            // local map size
     double *zmap;             // pass 1: output;  pass 2: the binned map;  fused: unused
-    const double *cov;        // fused: [n_pix, 6]
+    const double *cov;        // fused: [n_pix, nnz (nnz + 1) / 2]
     int accumulate;           // pass 1: add to zmap (REDs) even for single-unit blocks
 };
 
@@ -199,14 +202,14 @@ struct BxRec {
     int2 r;     // {pixel | n0 << kBxShift | n1 << (kBxShift + 6), slot}
     double2 qu; // (sum Q, sum U)
 };
-template <bool KEEP_IN_L2>
+template <bool KEEP_IN_L2, int NNZ>
 __device__ __forceinline__ BxRec bx_load(const BxArgs &a, int i, int end, int lane) {
     BxRec x;
     x.r = make_int2(0, -1 - lane); // idle lanes: n0 = n1 = 0, distinct negative slots
     x.qu = make_double2(0.0, 0.0);
     if (i < end) {
         x.r = KEEP_IN_L2 ? __ldg(a.brec + i) : __ldcs(a.brec + i);
-        x.qu = KEEP_IN_L2 ? __ldg(a.bqu + i) : __ldcs(a.bqu + i);
+        if constexpr (NNZ == 3) x.qu = KEEP_IN_L2 ? __ldg(a.bqu + i) : __ldcs(a.bqu + i);
     }
     return x;
 }
@@ -243,7 +246,8 @@ __device__ __forceinline__ double4 bx_consts(const BxArgs &a, int32_t slot) {
 }
 
 // one pass-1 step: the 32 records of `x` (amplitudes already gathered in `g`) into the tile
-template <bool UNIFORM, bool PAIRED>
+// (NNZ = 1: the tile holds one value per pixel and only the first term is formed)
+template <bool UNIFORM, bool PAIRED, int NNZ>
 __device__ __forceinline__ void bx_acc_step(const BxArgs &a, double *tile, const BxRec &x,
                                             const BxAmp &g, int lane) {
     const int p = x.r.x & (kBxPix - 1);
@@ -260,20 +264,24 @@ __device__ __forceinline__ void bx_acc_step(const BxArgs &a, double *tile, const
     const unsigned same = __match_any_sync(0xffffffffu, contrib ? p : kBxPix + lane);
     const int rank = __popc(same & ((1u << lane) - 1u));
     const int rounds = __reduce_max_sync(0xffffffffu, rank);
-    double *z = tile + 3 * p;
+    double *z = tile + NNZ * p;
     if (rounds == 0) {
         if (contrib) {
             z[0] += v0;
-            z[1] += v1;
-            z[2] += v2;
+            if constexpr (NNZ == 3) {
+                z[1] += v1;
+                z[2] += v2;
+            }
         }
         __syncwarp();
     } else {
         for (int r = 0; r <= rounds; ++r) {
             if (contrib && rank == r) {
                 z[0] += v0;
-                z[1] += v1;
-                z[2] += v2;
+                if constexpr (NNZ == 3) {
+                    z[1] += v1;
+                    z[2] += v2;
+                }
             }
             __syncwarp();
         }
@@ -283,50 +291,55 @@ __device__ __forceinline__ void bx_acc_step(const BxArgs &a, double *tile, const
 // pass 1 over the records [first, end) of the warp's unit: tile += a w (n cal, sum Q, sum U).
 // Software pipeline without register rotation (three record buffers, loop unrolled by three):
 // records are loaded two steps ahead, amplitudes gathered one step ahead.
-template <bool UNIFORM, bool PAIRED, bool KEEP_IN_L2>
+template <bool UNIFORM, bool PAIRED, bool KEEP_IN_L2, int NNZ>
 __device__ __forceinline__ void bx_accumulate(const BxArgs &a, double *tile, int first, int end,
                                               int lane) {
     if (first >= end) return;
-    BxRec A = bx_load<KEEP_IN_L2>(a, first + lane, end, lane);
-    BxRec B = bx_load<KEEP_IN_L2>(a, first + 32 + lane, end, lane);
+    BxRec A = bx_load<KEEP_IN_L2, NNZ>(a, first + lane, end, lane);
+    BxRec B = bx_load<KEEP_IN_L2, NNZ>(a, first + 32 + lane, end, lane);
     BxRec C;
     BxAmp gA = bx_gather<PAIRED, false>(a, A.r.y), gB, gC;
     for (int base = first; base < end; base += 96) {
-        C = bx_load<KEEP_IN_L2>(a, base + 64 + lane, end, lane);
+        C = bx_load<KEEP_IN_L2, NNZ>(a, base + 64 + lane, end, lane);
         gB = bx_gather<PAIRED, false>(a, B.r.y);
-        bx_acc_step<UNIFORM, PAIRED>(a, tile, A, gA, lane);
+        bx_acc_step<UNIFORM, PAIRED, NNZ>(a, tile, A, gA, lane);
         if (base + 32 >= end) break;
-        A = bx_load<KEEP_IN_L2>(a, base + 96 + lane, end, lane);
+        A = bx_load<KEEP_IN_L2, NNZ>(a, base + 96 + lane, end, lane);
         gC = bx_gather<PAIRED, false>(a, C.r.y);
-        bx_acc_step<UNIFORM, PAIRED>(a, tile, B, gB, lane);
+        bx_acc_step<UNIFORM, PAIRED, NNZ>(a, tile, B, gB, lane);
         if (base + 64 >= end) break;
-        B = bx_load<KEEP_IN_L2>(a, base + 128 + lane, end, lane);
+        B = bx_load<KEEP_IN_L2, NNZ>(a, base + 128 + lane, end, lane);
         gA = bx_gather<PAIRED, false>(a, A.r.y);
-        bx_acc_step<UNIFORM, PAIRED>(a, tile, C, gC, lane);
+        bx_acc_step<UNIFORM, PAIRED, NNZ>(a, tile, C, gC, lane);
     }
 }
 
 // one pass-2 step: out[baseline] += w (n a - (n cal, sum Q, sum U) . m), one RED pair per run of
 // records that share the baseline (consecutive in (row, time) order)
-template <bool UNIFORM, bool PAIRED>
+template <bool UNIFORM, bool PAIRED, int NNZ>
 __device__ __forceinline__ void bx_proj_step(const BxArgs &a, const double *tile, const BxRec &x,
                                              const BxAmp &g, int lane) {
     const int p = x.r.x & (kBxPix - 1);
     const int n0 = (x.r.x >> kBxShift) & 63, n1 = (x.r.x >> (kBxShift + 6)) & 63;
     const double4 c = bx_consts<UNIFORM>(a, x.r.y);
-    const double m0 = tile[3 * p], m1 = tile[3 * p + 1], m2 = tile[3 * p + 2];
+    const double m0 = tile[NNZ * p];
+    const double m1 = NNZ == 3 ? tile[NNZ * p + 1] : 0.0, m2 = NNZ == 3 ? tile[NNZ * p + 2] : 0.0;
     double val0 = 0.0, val1 = 0.0;
     if (n0) {
         double sc = (c.x * (double)n0) * m0;
-        sc += x.qu.x * m1;
-        sc += x.qu.y * m2;
+        if constexpr (NNZ == 3) {
+            sc += x.qu.x * m1;
+            sc += x.qu.y * m2;
+        }
         val0 = (double)n0 * g.t.x - sc * g.w.x;
     }
     if (PAIRED && n1) {
         const double q1 = c.z * x.qu.x - c.w * x.qu.y, u1 = c.w * x.qu.x + c.z * x.qu.y;
         double sc = (c.y * (double)n1) * m0;
-        sc += q1 * m1;
-        sc += u1 * m2;
+        if constexpr (NNZ == 3) {
+            sc += q1 * m1;
+            sc += u1 * m2;
+        }
         val1 = (double)n1 * g.t.y - sc * g.w.y;
     }
     const Runs rr = find_runs32<8>(x.r.y, lane);
@@ -341,39 +354,40 @@ __device__ __forceinline__ void bx_proj_step(const BxArgs &a, const double *tile
     }
 }
 
-template <bool UNIFORM, bool PAIRED>
+template <bool UNIFORM, bool PAIRED, int NNZ>
 __device__ __forceinline__ void bx_project(const BxArgs &a, const double *tile, int first, int end,
                                            int lane) {
     if (first >= end) return;
-    BxRec A = bx_load<false>(a, first + lane, end, lane);
-    BxRec B = bx_load<false>(a, first + 32 + lane, end, lane);
+    BxRec A = bx_load<false, NNZ>(a, first + lane, end, lane);
+    BxRec B = bx_load<false, NNZ>(a, first + 32 + lane, end, lane);
     BxRec C;
     BxAmp gA = bx_gather<PAIRED, true>(a, A.r.y), gB, gC;
     for (int base = first; base < end; base += 96) {
-        C = bx_load<false>(a, base + 64 + lane, end, lane);
+        C = bx_load<false, NNZ>(a, base + 64 + lane, end, lane);
         gB = bx_gather<PAIRED, true>(a, B.r.y);
-        bx_proj_step<UNIFORM, PAIRED>(a, tile, A, gA, lane);
+        bx_proj_step<UNIFORM, PAIRED, NNZ>(a, tile, A, gA, lane);
         if (base + 32 >= end) break;
-        A = bx_load<false>(a, base + 96 + lane, end, lane);
+        A = bx_load<false, NNZ>(a, base + 96 + lane, end, lane);
         gC = bx_gather<PAIRED, true>(a, C.r.y);
-        bx_proj_step<UNIFORM, PAIRED>(a, tile, B, gB, lane);
+        bx_proj_step<UNIFORM, PAIRED, NNZ>(a, tile, B, gB, lane);
         if (base + 64 >= end) break;
-        B = bx_load<false>(a, base + 128 + lane, end, lane);
+        B = bx_load<false, NNZ>(a, base + 128 + lane, end, lane);
         gA = bx_gather<PAIRED, true>(a, A.r.y);
-        bx_proj_step<UNIFORM, PAIRED>(a, tile, C, gC, lane);
+        bx_proj_step<UNIFORM, PAIRED, NNZ>(a, tile, C, gC, lane);
     }
 }
 
 // MODE 0: pass 1 (tile -> zmap), 1: pass 2 (binned map -> tile -> amplitudes), 2: fused.
 // One warp per work unit, eight consecutive units per CTA; grid = ceil(n_units / 8).
-template <int MODE, bool UNIFORM, bool PAIRED>
+// NNZ: map values per pixel, 3 (I, Q, U) or 1 (intensity: the map is [n_pix], cov [n_pix]).
+template <int MODE, bool UNIFORM, bool PAIRED, int NNZ>
 __global__ void __launch_bounds__(kThreads, TB_BX_CTAS)
 k_bx(const BxArgs a, int64_t n_units) {
-    __shared__ __align__(16) double tiles[kBxWarps][3 * kBxPix];
+    __shared__ __align__(16) double tiles[kBxWarps][NNZ * kBxPix];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     double *tile = tiles[warp];
     double2 *tile2 = reinterpret_cast<double2 *>(tile);
-    const int64_t g_end = 3 * a.n_pix;
+    const int64_t g_end = NNZ * a.n_pix;
     // (persistent warps taking tickets from a global counter measured slower than this static
     // assignment -- 0.88 vs 0.78 ms for the fused kernel on the C4 shard, profiles/README.md:
     // concurrently running neighbours share their amplitude sectors in the L1 / L2)
@@ -381,12 +395,12 @@ k_bx(const BxArgs a, int64_t n_units) {
         const int64_t ticket = (int64_t)blockIdx.x * kBxWarps + warp;
         if (ticket >= n_units) return;
         const int4 u = __ldg(a.units + ticket);
-        const int64_t g0 = (int64_t)u.x * (3 * kBxPix);      // first map double of the block
+        const int64_t g0 = (int64_t)u.x * (NNZ * kBxPix);    // first map double of the block
         if constexpr (MODE == 1) {
             if (u.z <= u.y) return; // nothing to project from this block
             const double2 *src = reinterpret_cast<const double2 *>(a.zmap + g0);
 #pragma unroll 4
-            for (int k = lane; k < 3 * kBxPix / 2; k += 32) {
+            for (int k = lane; k < NNZ * kBxPix / 2; k += 32) {
                 const int64_t g = g0 + 2 * k;
                 double2 v = make_double2(0.0, 0.0);
                 if (g + 1 < g_end) v = __ldcs(src + k);
@@ -394,53 +408,63 @@ k_bx(const BxArgs a, int64_t n_units) {
                 tile2[k] = v;
             }
             __syncwarp();
-            bx_project<UNIFORM, PAIRED>(a, tile, u.y, u.z, lane);
+            bx_project<UNIFORM, PAIRED, NNZ>(a, tile, u.y, u.z, lane);
         } else {
 #pragma unroll 4
-            for (int k = lane; k < 3 * kBxPix / 2; k += 32) tile2[k] = make_double2(0.0, 0.0);
+            for (int k = lane; k < NNZ * kBxPix / 2; k += 32) tile2[k] = make_double2(0.0, 0.0);
             __syncwarp();
-            bx_accumulate<UNIFORM, PAIRED, MODE == 2>(a, tile, u.y, u.z, lane);
+            bx_accumulate<UNIFORM, PAIRED, MODE == 2, NNZ>(a, tile, u.y, u.z, lane);
             __syncwarp();
             if constexpr (MODE == 0) {
                 if (u.w == 0 && !a.accumulate) {
                     // the only unit of its block: the tile IS the block of the map
                     double2 *dst = reinterpret_cast<double2 *>(a.zmap + g0);
 #pragma unroll 4
-                    for (int k = lane; k < 3 * kBxPix / 2; k += 32) {
+                    for (int k = lane; k < NNZ * kBxPix / 2; k += 32) {
                         const int64_t gg = g0 + 2 * k;
                         if (gg + 1 < g_end) __stcs(dst + k, tile2[k]);
                         else if (gg < g_end) a.zmap[gg] = tile2[k].x;
                     }
                 } else {
-                    for (int k = lane; k < 3 * kBxPix; k += 32) {
+                    for (int k = lane; k < NNZ * kBxPix; k += 32) {
                         const double v = tile[k];
                         if (v != 0.0 && g0 + k < g_end) atomicAdd(a.zmap + g0 + k, v);
                     }
                 }
             } else if (u.z > u.y) {
-                // fused: m = C z in place (toast_map_cov.cpp:509-517 operation order)
-                for (int p = lane; p < kBxPix; p += 32) {
-                    const int64_t gp = (int64_t)u.x * kBxPix + p;
-                    const double z0 = tile[3 * p], z1 = tile[3 * p + 1], z2 = tile[3 * p + 2];
-                    if (gp >= a.n_pix || (z0 == 0.0 && z1 == 0.0 && z2 == 0.0)) continue;
-                    const double2 *cm = reinterpret_cast<const double2 *>(a.cov + 6 * gp);
-                    const double2 ca = __ldcs(cm), cb = __ldcs(cm + 1), cc = __ldcs(cm + 2);
-                    double m0 = 0.0, m1 = 0.0, m2 = 0.0;
-                    m0 += ca.x * z0;
-                    m0 += ca.y * z1;
-                    m1 += ca.y * z0;
-                    m0 += cb.x * z2;
-                    m2 += cb.x * z0;
-                    m1 += cb.y * z1;
-                    m1 += cc.x * z2;
-                    m2 += cc.x * z1;
-                    m2 += cc.y * z2;
-                    tile[3 * p] = m0;
-                    tile[3 * p + 1] = m1;
-                    tile[3 * p + 2] = m2;
+                if constexpr (NNZ == 1) {
+                    // fused: m = C z in place (toast_map_cov.cpp:471-528, the nnz == 1 branch)
+                    for (int p = lane; p < kBxPix; p += 32) {
+                        const int64_t gp = (int64_t)u.x * kBxPix + p;
+                        const double z0 = tile[p];
+                        if (gp >= a.n_pix || z0 == 0.0) continue;
+                        tile[p] = z0 * __ldcs(a.cov + gp);
+                    }
+                } else {
+                    // fused: m = C z in place (toast_map_cov.cpp:509-517 operation order)
+                    for (int p = lane; p < kBxPix; p += 32) {
+                        const int64_t gp = (int64_t)u.x * kBxPix + p;
+                        const double z0 = tile[3 * p], z1 = tile[3 * p + 1], z2 = tile[3 * p + 2];
+                        if (gp >= a.n_pix || (z0 == 0.0 && z1 == 0.0 && z2 == 0.0)) continue;
+                        const double2 *cm = reinterpret_cast<const double2 *>(a.cov + 6 * gp);
+                        const double2 ca = __ldcs(cm), cb = __ldcs(cm + 1), cc = __ldcs(cm + 2);
+                        double m0 = 0.0, m1 = 0.0, m2 = 0.0;
+                        m0 += ca.x * z0;
+                        m0 += ca.y * z1;
+                        m1 += ca.y * z0;
+                        m0 += cb.x * z2;
+                        m2 += cb.x * z0;
+                        m1 += cb.y * z1;
+                        m1 += cc.x * z2;
+                        m2 += cc.x * z1;
+                        m2 += cc.y * z2;
+                        tile[3 * p] = m0;
+                        tile[3 * p + 1] = m1;
+                        tile[3 * p + 2] = m2;
+                    }
                 }
                 __syncwarp();
-                bx_project<UNIFORM, PAIRED>(a, tile, u.y, u.z, lane);
+                bx_project<UNIFORM, PAIRED, NNZ>(a, tile, u.y, u.z, lane);
             }
         }
     }
@@ -448,13 +472,15 @@ k_bx(const BxArgs a, int64_t n_units) {
 
 // zero / covariance product on whole blocks of the global map (the multi-unit blocks of the fused
 // path: their units meet in global memory)
+template <int NNZ>
 __global__ void __launch_bounds__(kThreads)
 k_bx_zero_blocks(const int32_t *__restrict__ blocks, int64_t n_pix, double *__restrict__ zmap) {
-    const int64_t g0 = (int64_t)__ldg(blocks + blockIdx.x) * (3 * kBxPix);
-    for (int k = threadIdx.x; k < 3 * kBxPix; k += kThreads)
-        if (g0 + k < 3 * n_pix) zmap[g0 + k] = 0.0;
+    const int64_t g0 = (int64_t)__ldg(blocks + blockIdx.x) * (NNZ * kBxPix);
+    for (int k = threadIdx.x; k < NNZ * kBxPix; k += kThreads)
+        if (g0 + k < NNZ * n_pix) zmap[g0 + k] = 0.0;
 }
 
+template <int NNZ>
 __global__ void __launch_bounds__(kThreads)
 k_bx_cov_blocks(const int32_t *__restrict__ blocks, int64_t n_pix, const double *__restrict__ cov,
                 double *__restrict__ zmap) {
@@ -462,22 +488,26 @@ k_bx_cov_blocks(const int32_t *__restrict__ blocks, int64_t n_pix, const double 
     for (int p = threadIdx.x; p < kBxPix; p += kThreads) {
         const int64_t gp = p0 + p;
         if (gp >= n_pix) continue;
-        double *z = zmap + 3 * gp;
-        const double z0 = z[0], z1 = z[1], z2 = z[2];
-        const double *m = cov + 6 * gp;
-        double t0 = 0.0, t1 = 0.0, t2 = 0.0;
-        t0 += m[0] * z0;
-        t0 += m[1] * z1;
-        t1 += m[1] * z0;
-        t0 += m[2] * z2;
-        t2 += m[2] * z0;
-        t1 += m[3] * z1;
-        t1 += m[4] * z2;
-        t2 += m[4] * z1;
-        t2 += m[5] * z2;
-        z[0] = t0;
-        z[1] = t1;
-        z[2] = t2;
+        if constexpr (NNZ == 1) {
+            zmap[gp] = zmap[gp] * cov[gp];
+        } else {
+            double *z = zmap + 3 * gp;
+            const double z0 = z[0], z1 = z[1], z2 = z[2];
+            const double *m = cov + 6 * gp;
+            double t0 = 0.0, t1 = 0.0, t2 = 0.0;
+            t0 += m[0] * z0;
+            t0 += m[1] * z1;
+            t1 += m[1] * z0;
+            t0 += m[2] * z2;
+            t2 += m[2] * z0;
+            t1 += m[3] * z1;
+            t1 += m[4] * z2;
+            t2 += m[4] * z1;
+            t2 += m[5] * z2;
+            z[0] = t0;
+            z[1] = t1;
+            z[2] = t2;
+        }
     }
 }
 
@@ -518,32 +548,49 @@ void launch_bx_prescale(const tb_obs *obs, const double *amps, const uint8_t *af
     tbr::count_launch();
 }
 
-template <int MODE>
-void launch_bx(const tb_obs *obs, const BxArgs &a, int64_t n_units, void *stream) {
-    if (n_units <= 0) return;
+template <int MODE, int NNZ>
+void launch_bx_nnz(const tb_obs *obs, const BxArgs &a, int64_t n_units, void *stream) {
     const int64_t nb = (n_units + kBxWarps - 1) / kBxWarps;
     TB_REQUIRE(nb < 2147483647LL, "grid too large");
     const unsigned g = (unsigned)nb;
     cudaStream_t st = (cudaStream_t)stream;
-    static bool configured = false; // (per MODE instantiation)
+    static bool configured = false; // (per MODE / NNZ instantiation)
     if (!configured) {
         auto prep = [&](const void *f) {
             TB_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout,
                                          (int)cudaSharedmemCarveoutMaxShared));
         };
-        prep((const void *)k_bx<MODE, true, true>);
-        prep((const void *)k_bx<MODE, true, false>);
-        prep((const void *)k_bx<MODE, false, true>);
-        prep((const void *)k_bx<MODE, false, false>);
+        prep((const void *)k_bx<MODE, true, true, NNZ>);
+        prep((const void *)k_bx<MODE, true, false, NNZ>);
+        prep((const void *)k_bx<MODE, false, true, NNZ>);
+        prep((const void *)k_bx<MODE, false, false, NNZ>);
         configured = true;
     }
     if (obs->s_uniform) {
-        if (obs->x_paired) k_bx<MODE, true, true><<<g, kThreads, 0, st>>>(a, n_units);
-        else k_bx<MODE, true, false><<<g, kThreads, 0, st>>>(a, n_units);
+        if (obs->x_paired) k_bx<MODE, true, true, NNZ><<<g, kThreads, 0, st>>>(a, n_units);
+        else k_bx<MODE, true, false, NNZ><<<g, kThreads, 0, st>>>(a, n_units);
     } else {
-        if (obs->x_paired) k_bx<MODE, false, true><<<g, kThreads, 0, st>>>(a, n_units);
-        else k_bx<MODE, false, false><<<g, kThreads, 0, st>>>(a, n_units);
+        if (obs->x_paired) k_bx<MODE, false, true, NNZ><<<g, kThreads, 0, st>>>(a, n_units);
+        else k_bx<MODE, false, false, NNZ><<<g, kThreads, 0, st>>>(a, n_units);
     }
+    TB_CUDA(cudaGetLastError());
+    tbr::count_launch();
+}
+
+template <int MODE>
+void launch_bx(const tb_obs *obs, const BxArgs &a, int64_t n_units, void *stream) {
+    if (n_units <= 0) return;
+    if (obs->nnz == 1) launch_bx_nnz<MODE, 1>(obs, a, n_units, stream);
+    else launch_bx_nnz<MODE, 3>(obs, a, n_units, stream);
+}
+
+void launch_zero_blocks(const tb_obs *obs, double *zmap, cudaStream_t st) {
+    if (obs->nnz == 1)
+        k_bx_zero_blocks<1><<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
+            obs->bmulti_blocks, obs->n_local_pix, zmap);
+    else
+        k_bx_zero_blocks<3><<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
+            obs->bmulti_blocks, obs->n_local_pix, zmap);
     TB_CUDA(cudaGetLastError());
     tbr::count_launch();
 }
@@ -637,16 +684,22 @@ void tb_build_blocked(tb_obs *obs, cudaStream_t st) {
         kin = vin = nullptr;
         // (two records of padding: the staged copies start / end on even record indices)
         TB_CUDA(cudaMalloc(&obs->brec, sizeof(int2) * (n_sorted + 2)));
-        TB_CUDA(cudaMalloc(&obs->bqu, sizeof(double2) * (n_sorted + 2)));
         TB_CUDA(cudaMemsetAsync(obs->brec + n_sorted, 0, sizeof(int2) * 2, st));
-        TB_CUDA(cudaMemsetAsync(obs->bqu + n_sorted, 0, sizeof(double2) * 2, st));
+        if (obs->nnz == 3) {
+            TB_CUDA(cudaMalloc(&obs->bqu, sizeof(double2) * (n_sorted + 2)));
+            TB_CUDA(cudaMemsetAsync(obs->bqu + n_sorted, 0, sizeof(double2) * 2, st));
+        }
         {
             const size_t slots = (size_t)obs->n_xrows * (size_t)nad;
             const size_t per = obs->x_paired ? 2 : 1;
             TB_CUDA(cudaMalloc(&obs->ascaled, sizeof(double) * 2 * per * slots));
         }
-        k_bx_gather<<<grid, kThreads, 0, st>>>(obs->xrec, obs->xqu, vout, n_sorted, nad, 1,
-                                               obs->brec, obs->bqu);
+        if (obs->nnz == 1)
+            k_bx_gather<1><<<grid, kThreads, 0, st>>>(obs->xrec, nullptr, vout, n_sorted, nad, 1,
+                                                      obs->brec, nullptr);
+        else
+            k_bx_gather<3><<<grid, kThreads, 0, st>>>(obs->xrec, obs->xqu, vout, n_sorted, nad,
+                                                      1, obs->brec, obs->bqu);
         TB_CUDA(cudaGetLastError());
         tbr::count_launch();
         TB_CUDA(cudaMalloc(&starts, sizeof(int32_t) * (n_blocks + 1)));
@@ -752,10 +805,7 @@ int tb_bx_pass1(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_
     if (chunk <= 0) launch_bx_prescale(obs, amplitudes, amp_flags, stream);
     if (!accumulate && obs->n_bmulti_blocks > 0 && chunk <= 0) {
         // the units of a multi-unit block meet in global memory: it starts from zero
-        k_bx_zero_blocks<<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, (cudaStream_t)stream>>>(
-            obs->bmulti_blocks, obs->n_local_pix, zmap);
-        TB_CUDA(cudaGetLastError());
-        tbr::count_launch();
+        launch_zero_blocks(obs, zmap, (cudaStream_t)stream);
     }
     BxArgs a = make_args(obs, obs->bunits + first);
     a.zmap = zmap;
@@ -798,15 +848,16 @@ int tb_bx_fused(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_
         TB_REQUIRE(zmap_scratch != nullptr, "blocks with several units need the zmap scratch");
         TB_REQUIRE((reinterpret_cast<uintptr_t>(zmap_scratch) & 15u) == 0,
                    "zmap scratch must be 16-byte aligned");
-        k_bx_zero_blocks<<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
-            obs->bmulti_blocks, obs->n_local_pix, zmap_scratch);
-        TB_CUDA(cudaGetLastError());
-        tbr::count_launch();
+        launch_zero_blocks(obs, zmap_scratch, st);
         BxArgs m = make_args(obs, obs->bunits_multi);
         m.zmap = zmap_scratch;
         launch_bx<0>(obs, m, obs->n_bunits_multi, stream);
-        k_bx_cov_blocks<<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
-            obs->bmulti_blocks, obs->n_local_pix, cov, zmap_scratch);
+        if (obs->nnz == 1)
+            k_bx_cov_blocks<1><<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
+                obs->bmulti_blocks, obs->n_local_pix, cov, zmap_scratch);
+        else
+            k_bx_cov_blocks<3><<<(unsigned)obs->n_bmulti_blocks, kThreads, 0, st>>>(
+                obs->bmulti_blocks, obs->n_local_pix, cov, zmap_scratch);
         TB_CUDA(cudaGetLastError());
         tbr::count_launch();
         m.out = amplitudes_out;

@@ -26,6 +26,10 @@ struct tb_obs {
     tb_obs_desc d; // copy of the descriptor (host pointers in it are NOT kept alive)
     int is_wcs = 0; // pixels of a flat projection (tb_obs_create_wcs): regenerated with `wcs`
     tbw::Wcs wcs{};
+    // Stokes values per pixel: 3 (I, Q, U; weights [n_det, n_samp, 3]) or 1 (intensity only,
+    // tb_obs_create_intensity; weights [n_det, n_samp] = cal[det]).  Intensity observations
+    // keep no (Q, U) arrays: wqu, xqu and bqu stay NULL, and lpp / pair_rot are never built.
+    int nnz = 3;
     int64_t n_amp_det = 0;
     // compact solver pointing (tb_obs_pack_pointing): local pixel (int32, <0 = nothing to do)
     // and the two sample-dependent weights (Q, U) as one 16-byte record
@@ -42,7 +46,7 @@ struct tb_obs {
     int4 *xblocks = nullptr;    // [n_xblocks] {row, first record, end record, 0}
     int64_t n_xrec = 0, n_xblocks = 0, n_xrows = 0;
     int x_paired = 0;           // rows are detector pairs (weights shared through pair_rot)
-    double4 *stable = nullptr;  // [n_xrows] {cal0, cal1, A, B}
+    double4 *stable = nullptr;  // [n_xrows] {cal0, cal1, A, B} (A = B = 0 for intensity)
     // block-ordered crossing list (tb_blocked.cu): the time-ordered records stably sorted by
     // PIXEL BLOCK (kBxPix consecutive local pixels), i.e. in (block, row, time) order.  A CTA owns
     // one block at a time and keeps its 3 x kBxPix map values in shared memory.

@@ -58,18 +58,25 @@ __device__ unsigned long long g_exact_count_solver = 0ull;
 constexpr int kBinRunCap = TB_BIN_RUN_CAP; // see find_runs<CAP>
 
 // pixel + weights of one sample, either streamed from HBM or regenerated from the boresight with
-// the pixelisation policy PIX (tb_pixelise.cuh: the device function tb_pointing_fused[_wcs] runs)
-template <bool REGEN, class PIX>
+// the pixelisation policy PIX (tb_pixelise.cuh: the device function tb_pointing_fused[_wcs] runs).
+// NNZ = 1: the intensity weight alone (stored [n_det, n_samp], or cal[det] as
+// ops_stokes_weights.cpp's I mode sets it); w1 = w2 = 0.
+template <bool REGEN, class PIX, int NNZ>
 __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_t s, bool need,
                                                 int64_t &pix, double &w0, double &w1, double &w2,
                                                 int &n_exact) {
     if (!REGEN) {
         int64_t i = (int64_t)det * o.n_samp + s;
         pix = ld_stream(o.pixels + i);
-        const double *w = o.weights + 3 * i;
-        w0 = ld_stream(w);
-        w1 = ld_stream(w + 1);
-        w2 = ld_stream(w + 2);
+        if constexpr (NNZ == 1) {
+            w0 = ld_stream(o.weights + i);
+            w1 = w2 = 0.0;
+        } else {
+            const double *w = o.weights + 3 * i;
+            w0 = ld_stream(w);
+            w1 = ld_stream(w + 1);
+            w2 = ld_stream(w + 2);
+        }
     } else {
         pix = -1;
         w0 = w1 = w2 = 0.0;
@@ -81,6 +88,10 @@ __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_
             pix = PIX::pixel(o.wcs, q, n_exact);
         } else {
             pix = PIX::pixel(o.ctx, q, n_exact);
+        }
+        if constexpr (NNZ == 1) {
+            w0 = __ldg(o.cal + det);
+            return;
         }
         double cal = __ldg(o.cal + det), eta = __ldg(o.eta + det);
         if (o.hwp) {
@@ -113,10 +124,11 @@ __device__ __forceinline__ void sample_pointing(const ObsDev &o, int det, int64_
 
 // ---- pass 1: template -> timestream -> noise-weighted map -------------------------------------
 // FROM_SIGNAL: bin a stored timestream instead of the template amplitudes (RHS / final BinMap).
+// NNZ: map values per pixel, 3 (I, Q, U) or 1 (intensity).
 #ifndef TB_REGEN_CTAS
 #define TB_REGEN_CTAS 4
 #endif
-template <bool REGEN, class PIX, bool FROM_SIGNAL>
+template <bool REGEN, class PIX, bool FROM_SIGNAL, int NNZ>
 __global__ void __launch_bounds__(kThreads, REGEN ? TB_REGEN_CTAS : 6)
 k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ aflags,
       const double *__restrict__ signal, double *__restrict__ zmap) {
@@ -138,7 +150,7 @@ k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ afl
             }
             int64_t pix;
             double w0, w1, w2;
-            sample_pointing<REGEN, PIX>(o, det, s, ok, pix, w0, w1, w2, n_exact);
+            sample_pointing<REGEN, PIX, NNZ>(o, det, s, ok, pix, w0, w1, w2, n_exact);
             if (ok && pix >= 0) {
                 int64_t gsm = fast_div(pix, o.inv_nps);
                 key = __ldg(o.g2l + gsm) * o.n_pix_submap + (pix - gsm * o.n_pix_submap);
@@ -150,20 +162,24 @@ k_bin(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ afl
         }
         Runs r = find_runs<kBinRunCap>(key, lane);
         z0 = seg_sum<kBinRunCap>(z0, r);
-        z1 = seg_sum<kBinRunCap>(z1, r);
-        z2 = seg_sum<kBinRunCap>(z2, r);
+        if constexpr (NNZ == 3) {
+            z1 = seg_sum<kBinRunCap>(z1, r);
+            z2 = seg_sum<kBinRunCap>(z2, r);
+        }
         if (r.is_tail && key >= 0) {
-            double *z = zmap + key * 3;
+            double *z = zmap + key * NNZ;
             atomicAdd(z, z0);
-            atomicAdd(z + 1, z1);
-            atomicAdd(z + 2, z2);
+            if constexpr (NNZ == 3) {
+                atomicAdd(z + 1, z1);
+                atomicAdd(z + 2, z2);
+            }
         }
     }
     if (REGEN && n_exact) atomicAdd(&g_exact_count_solver, (unsigned long long)n_exact);
 }
 
 // ---- pass 2: (template - scanned map) -> noise weight -> template projection ------------------
-template <bool REGEN, class PIX, bool FROM_SIGNAL>
+template <bool REGEN, class PIX, bool FROM_SIGNAL, int NNZ>
 __global__ void __launch_bounds__(kThreads, REGEN ? TB_REGEN_CTAS : 6)
 k_project(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__ aflags,
           const double *__restrict__ signal, const double *__restrict__ binned,
@@ -191,16 +207,18 @@ k_project(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__
             }
             int64_t pix;
             double w0, w1, w2;
-            sample_pointing<REGEN, PIX>(o, det, s, need, pix, w0, w1, w2, n_exact);
+            sample_pointing<REGEN, PIX, NNZ>(o, det, s, need, pix, w0, w1, w2, n_exact);
             if (need) {
                 if (pix >= 0) {
                     int64_t gsm = fast_div(pix, o.inv_nps);
-                    const double *m = binned + 3 * (__ldg(o.g2l + gsm) * o.n_pix_submap +
-                                                    (pix - gsm * o.n_pix_submap));
+                    const double *m = binned + NNZ * (__ldg(o.g2l + gsm) * o.n_pix_submap +
+                                                      (pix - gsm * o.n_pix_submap));
                     double sc = 0.0; // ops_scan_map.cpp:59-64
                     sc += w0 * __ldg(m);
-                    sc += w1 * __ldg(m + 1);
-                    sc += w2 * __ldg(m + 2);
+                    if constexpr (NNZ == 3) {
+                        sc += w1 * __ldg(m + 1);
+                        sc += w2 * __ldg(m + 2);
+                    }
                     tod -= sc;
                 }
                 v = tod * __ldg(o.det_scale + det);
@@ -228,6 +246,8 @@ k_project(ObsDev o, const double *__restrict__ amps, const uint8_t *__restrict__
 // =================================================================================================
 __device__ unsigned int g_pack_mismatch = 0u;
 
+// NNZ = 1: intensity weights [n_det, n_samp]; only lpix is written (the 4-byte form)
+template <int NNZ>
 __global__ void __launch_bounds__(kThreads)
 k_pack_pointing(ObsDev o, int32_t *__restrict__ lpix, double2 *__restrict__ wqu) {
     const int64_t total = o.n_det * o.n_samp;
@@ -236,8 +256,15 @@ k_pack_pointing(ObsDev o, int32_t *__restrict__ lpix, double2 *__restrict__ wqu)
          i += (int64_t)gridDim.x * kThreads) {
         int det = (int)(i / o.n_samp);
         int64_t pix = ld_stream(o.pixels + i);
-        const double *w = o.weights + 3 * i;
-        double w0 = ld_stream(w), w1 = ld_stream(w + 1), w2 = ld_stream(w + 2);
+        double w0, w1 = 0.0, w2 = 0.0;
+        if constexpr (NNZ == 1) {
+            w0 = ld_stream(o.weights + i);
+        } else {
+            const double *w = o.weights + 3 * i;
+            w0 = ld_stream(w);
+            w1 = ld_stream(w + 1);
+            w2 = ld_stream(w + 2);
+        }
         bool ok = o.solver_flags ? ((ld_stream(o.solver_flags + i) & o.solver_mask) == 0) : true;
         int32_t lp = -1;
         if (ok) {
@@ -252,7 +279,7 @@ k_pack_pointing(ObsDev o, int32_t *__restrict__ lpix, double2 *__restrict__ wqu)
             }
         }
         lpix[i] = lp;
-        wqu[i] = make_double2(w1, w2);
+        if constexpr (NNZ == 3) wqu[i] = make_double2(w1, w2);
     }
     if (bad) atomicOr(&g_pack_mismatch, 1u);
 }
@@ -623,7 +650,9 @@ struct XState {
     double2 wq;
 };
 
-// state of flat sample t of row `row` (a detector pair when paired, else one detector)
+// state of flat sample t of row `row` (a detector pair when paired, else one detector);
+// NNZ = 1 reads no (Q, U) weights
+template <int NNZ>
 __device__ __forceinline__ XState x_state(const ObsDev &o, int paired, int64_t row, int64_t t) {
     XState st;
     st.lp0 = st.lp1 = -1;
@@ -636,14 +665,17 @@ __device__ __forceinline__ XState x_state(const ObsDev &o, int paired, int64_t r
     int64_t d0 = paired ? 2 * row : row;
     int64_t i0 = d0 * o.n_samp + s;
     st.lp0 = __ldcs(o.lpix + i0);
-    st.wq = __ldcs(o.wqu + i0);
+    if constexpr (NNZ == 3) st.wq = __ldcs(o.wqu + i0);
     if (paired && d0 + 1 < o.n_det) st.lp1 = __ldcs(o.lpix + i0 + o.n_samp);
     st.amp_rel = (int32_t)(__ldg(o.amp_view_off + view) + fast_div(off, o.inv_step));
     return st;
 }
 
-// FILL = false: counts[chunk] = records of the chunk; FILL = true: write them at base[chunk]
-template <bool FILL>
+// FILL = false: counts[chunk] = records of the chunk; FILL = true: write them at base[chunk].
+// NNZ = 1: intensity records (xrec only, no xqu).  Its counting pass on paired rows also adds
+// the records whose two detectors fall in different pixels (each takes two entries of the
+// block-ordered list) to counts[n_chunks], read as an unsigned counter.
+template <bool FILL, int NNZ>
 __global__ void __launch_bounds__(kThreads)
 k_xbuild(ObsDev o, int paired, int64_t n_rows, int64_t chunks_per_row, int32_t *__restrict__ counts,
          const int64_t *__restrict__ base, int4 *__restrict__ xrec, double2 *__restrict__ xqu) {
@@ -654,7 +686,7 @@ k_xbuild(ObsDev o, int paired, int64_t n_rows, int64_t chunks_per_row, int32_t *
     for (int64_t c = warp0; c < n_chunks; c += n_warps) {
         int64_t row = c / chunks_per_row;
         int64_t t = (c - row * chunks_per_row) * 32 + lane;
-        XState st = x_state(o, paired, row, t);
+        XState st = x_state<NNZ>(o, paired, row, t);
         int32_t p0 = __shfl_up_sync(0xffffffffu, st.lp0, 1);
         int32_t p1 = __shfl_up_sync(0xffffffffu, st.lp1, 1);
         int32_t pa = __shfl_up_sync(0xffffffffu, st.amp_rel, 1);
@@ -664,6 +696,15 @@ k_xbuild(ObsDev o, int paired, int64_t n_rows, int64_t chunks_per_row, int32_t *
         unsigned kept_heads = __ballot_sync(0xffffffffu, head && keep);
         if (!FILL) {
             if (lane == 0) counts[c] = __popc(kept_heads);
+            if constexpr (NNZ == 1) {
+                if (paired) {
+                    const unsigned split = __ballot_sync(
+                        0xffffffffu, head && st.lp0 >= 0 && st.lp1 >= 0 && st.lp0 != st.lp1);
+                    if (lane == 0 && split)
+                        atomicAdd(reinterpret_cast<unsigned int *>(counts + n_chunks),
+                                  (unsigned int)__popc(split));
+                }
+            }
             continue;
         }
         unsigned upto = heads & (0xffffffffu >> (31 - lane));
@@ -671,11 +712,15 @@ k_xbuild(ObsDev o, int paired, int64_t n_rows, int64_t chunks_per_row, int32_t *
         Runs r;
         r.dist = lane - head_lane;
         r.is_tail = (((heads >> 1) | 0x80000000u) >> lane) & 1u;
-        double Q = seg_sum(st.wq.x, r), U = seg_sum(st.wq.y, r);
+        double Q = 0.0, U = 0.0;
+        if constexpr (NNZ == 3) {
+            Q = seg_sum(st.wq.x, r);
+            U = seg_sum(st.wq.y, r);
+        }
         if (r.is_tail && keep) {
             int64_t idx = base[c] + __popc(kept_heads & ((1u << head_lane) - 1u));
             xrec[idx] = make_int4(st.lp0, st.lp1, (r.dist + 1) | ((int)row << 8), st.amp_rel);
-            xqu[idx] = make_double2(Q, U);
+            if constexpr (NNZ == 3) xqu[idx] = make_double2(Q, U);
         }
     }
 }
@@ -864,12 +909,57 @@ inline int64_t obs_blocks(const tb_obs *obs) {
         }                                                                                  \
     } while (0)
 
+// the per-sample pass 1 (k_bin) with stored or regenerated pointing
+template <bool FROM_SIGNAL, int NNZ>
+void launch_bin_samples(const tb_obs *obs, const ObsDev &o, const double *amps,
+                        const uint8_t *aflags, const double *signal, double *zmap, int regen,
+                        void *stream) {
+    int64_t nb = obs_blocks(obs);
+    if (!regen) {
+        auto k = k_bin<false, tbp::PixHealpix<true>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+    } else if (obs->is_wcs) {
+        auto k = k_bin<true, tbp::PixWcs, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+    } else if (obs->d.nest) {
+        auto k = k_bin<true, tbp::PixHealpix<true>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+    } else {
+        auto k = k_bin<true, tbp::PixHealpix<false>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+    }
+}
+
+// the per-sample pass 2 (k_project) with stored or regenerated pointing
+template <bool FROM_SIGNAL, int NNZ>
+void launch_project_samples(const tb_obs *obs, const ObsDev &o, const double *amps,
+                            const uint8_t *aflags, const double *signal, const double *binned,
+                            double *out, int regen, void *stream) {
+    int64_t nb = obs_blocks(obs);
+    if (!regen) {
+        auto k = k_project<false, tbp::PixHealpix<true>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+    } else if (obs->is_wcs) {
+        auto k = k_project<true, tbp::PixWcs, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+    } else if (obs->d.nest) {
+        auto k = k_project<true, tbp::PixHealpix<true>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+    } else {
+        auto k = k_project<true, tbp::PixHealpix<false>, FROM_SIGNAL, NNZ>;
+        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+    }
+}
+
+// Intensity observations always take the per-sample kernels here: the crossing-list and
+// detector-pair kernels are IQU-only.
 template <bool FROM_SIGNAL>
 void launch_bin(const tb_obs *obs, const double *amps, const uint8_t *aflags, const double *signal,
                 double *zmap, int regen, void *stream) {
     ObsDev o = make_dev(obs, regen);
-    int64_t nb = obs_blocks(obs);
-    if (!regen && !FROM_SIGNAL && g_use_x && o.xrec != nullptr) {
+    if (obs->nnz == 1) {
+        launch_bin_samples<FROM_SIGNAL, 1>(obs, o, amps, aflags, signal, zmap, regen, stream);
+    } else if (!regen && !FROM_SIGNAL && g_use_x && o.xrec != nullptr) {
         auto k = k_lhs_x<false>;
         TBS_LAUNCH(k, obs->n_xblocks, stream, o, amps, aflags, nullptr, zmap);
     } else if (!regen && !FROM_SIGNAL && g_use_pair && o.lpix != nullptr) {
@@ -882,18 +972,8 @@ void launch_bin(const tb_obs *obs, const double *amps, const uint8_t *aflags, co
             auto k = k_lhs_pair<false>;
             TBS_LAUNCH(k, nbp, stream, o, n_pair, amps, aflags, nullptr, zmap);
         }
-    } else if (!regen) {
-        auto k = k_bin<false, tbp::PixHealpix<true>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
-    } else if (obs->is_wcs) {
-        auto k = k_bin<true, tbp::PixWcs, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
-    } else if (obs->d.nest) {
-        auto k = k_bin<true, tbp::PixHealpix<true>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
     } else {
-        auto k = k_bin<true, tbp::PixHealpix<false>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, zmap);
+        launch_bin_samples<FROM_SIGNAL, 3>(obs, o, amps, aflags, signal, zmap, regen, stream);
     }
 }
 
@@ -902,8 +982,10 @@ void launch_project(const tb_obs *obs, const double *amps, const uint8_t *aflags
                     const double *signal, const double *binned, double *out, int regen,
                     void *stream) {
     ObsDev o = make_dev(obs, regen);
-    int64_t nb = obs_blocks(obs);
-    if (!regen && !FROM_SIGNAL && g_use_x && o.xrec != nullptr) {
+    if (obs->nnz == 1) {
+        launch_project_samples<FROM_SIGNAL, 1>(obs, o, amps, aflags, signal, binned, out, regen,
+                                               stream);
+    } else if (!regen && !FROM_SIGNAL && g_use_x && o.xrec != nullptr) {
         auto k = k_lhs_x<true>;
         TBS_LAUNCH(k, obs->n_xblocks, stream, o, amps, aflags, binned, out);
     } else if (!regen && !FROM_SIGNAL && g_use_pair && o.lpix != nullptr) {
@@ -916,18 +998,9 @@ void launch_project(const tb_obs *obs, const double *amps, const uint8_t *aflags
             auto k = k_lhs_pair<true>;
             TBS_LAUNCH(k, nbp, stream, o, n_pair, amps, aflags, binned, out);
         }
-    } else if (!regen) {
-        auto k = k_project<false, tbp::PixHealpix<true>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
-    } else if (obs->is_wcs) {
-        auto k = k_project<true, tbp::PixWcs, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
-    } else if (obs->d.nest) {
-        auto k = k_project<true, tbp::PixHealpix<true>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
     } else {
-        auto k = k_project<true, tbp::PixHealpix<false>, FROM_SIGNAL>;
-        TBS_LAUNCH(k, nb, stream, o, amps, aflags, signal, binned, out);
+        launch_project_samples<FROM_SIGNAL, 3>(obs, o, amps, aflags, signal, binned, out, regen,
+                                               stream);
     }
 }
 
@@ -1054,8 +1127,9 @@ inline int red_grid(int64_t n) {
     return (int)b;
 }
 
-// the body of tb_obs_create / tb_obs_create_wcs; `wcs` NULL: a HEALPix observation
-tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
+// the body of tb_obs_create / tb_obs_create_wcs / tb_obs_create_intensity; `wcs` NULL: a HEALPix
+// observation
+tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs, int nnz) {
     try {
         tbr::require_device();
         TB_REQUIRE(desc != nullptr, "NULL descriptor");
@@ -1077,6 +1151,7 @@ tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
         o->d = d;
         o->is_wcs = wcs != nullptr;
         o->wcs = w;
+        o->nnz = nnz;
         // pack: int64 [first(nv), prefix(nv+1), amp_view_off(nv), amp_offsets(nd), g2l(ns)]
         //       double [fp(4nd), cal, eta, gamma, det_scale]
         int64_t nv = d.n_view, nd = d.n_det, ns = d.n_submap;
@@ -1145,15 +1220,21 @@ tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
 
 extern "C" {
 
-tb_obs *tb_obs_create(const tb_obs_desc *desc) { return obs_create(desc, nullptr); }
+tb_obs *tb_obs_create(const tb_obs_desc *desc) { return obs_create(desc, nullptr, 3); }
 
 tb_obs *tb_obs_create_wcs(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
     if (wcs == nullptr) {
         tbr::set_error(TB_ERR_ARG, "NULL projection");
         return nullptr;
     }
-    return obs_create(desc, wcs);
+    return obs_create(desc, wcs, 3);
 }
+
+tb_obs *tb_obs_create_intensity(const tb_obs_desc *desc, const tb_wcs_desc *wcs) {
+    return obs_create(desc, wcs, 1);
+}
+
+int tb_obs_nnz(const tb_obs *obs) { return obs ? obs->nnz : 0; }
 
 void tb_obs_destroy(tb_obs *obs) {
     if (obs == nullptr) return;
@@ -1183,9 +1264,10 @@ void tb_build_row_table(tb_obs *obs) {
     TB_CUDA(cudaMemcpy(cal.data(), obs->cal, sizeof(double) * n_det, cudaMemcpyDeviceToHost));
     std::vector<double2> rot;
     if (obs->x_paired) {
-        rot.resize(n_rows);
-        TB_CUDA(cudaMemcpy(rot.data(), obs->pair_rot, sizeof(double2) * n_rows,
-                           cudaMemcpyDeviceToHost));
+        rot.assign(n_rows, make_double2(0.0, 0.0)); // (intensity rows: no weight rotation)
+        if (obs->pair_rot)
+            TB_CUDA(cudaMemcpy(rot.data(), obs->pair_rot, sizeof(double2) * n_rows,
+                               cudaMemcpyDeviceToHost));
     }
     std::vector<double4> tab(n_rows);
     bool uniform = true;
@@ -1210,7 +1292,41 @@ void tb_build_row_table(tb_obs *obs) {
     obs->s_const[3] = tab[0].w;
 }
 
+// Records per 32-sample chunk of the crossing list in one row layout (the counting pass of
+// k_xbuild); for paired intensity rows also the records whose detectors fall in different pixels.
+static std::vector<int32_t> count_crossings(tb_obs *obs, int paired, int64_t n_rows, int64_t cpr,
+                                            int64_t *n_split, cudaStream_t st) {
+    const int64_t n_chunks = n_rows * cpr;
+    ObsDev o = make_dev(obs, 0);
+    int32_t *counts = nullptr;
+    TB_CUDA(cudaMalloc(&counts, sizeof(int32_t) * (n_chunks + 1)));
+    int grid = tbr::sm_count() * 8;
+    if (obs->nnz == 1) {
+        TB_CUDA(cudaMemsetAsync(counts + n_chunks, 0, sizeof(int32_t), st));
+        k_xbuild<false, 1><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, counts, nullptr,
+                                                      nullptr, nullptr);
+    } else {
+        k_xbuild<false, 3><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, counts, nullptr,
+                                                      nullptr, nullptr);
+    }
+    TB_CUDA(cudaGetLastError());
+    tbr::count_launch();
+    std::vector<int32_t> hc(n_chunks + 1, 0);
+    TB_CUDA(cudaMemcpyAsync(hc.data(), counts,
+                            sizeof(int32_t) * (obs->nnz == 1 ? n_chunks + 1 : n_chunks),
+                            cudaMemcpyDeviceToHost, st));
+    TB_CUDA(cudaStreamSynchronize(st));
+    cudaFree(counts);
+    if (n_split) *n_split = (int64_t)(uint32_t)hc[n_chunks];
+    hc.pop_back();
+    return hc;
+}
+
 // Collapse the packed pointing into the crossing list (k_lhs_x) when that is the smaller stream.
+// Intensity observations always get it (the block-ordered list is built from it), in the row
+// layout that gives the block-ordered list fewer entries: detector pairs share a record while
+// both detectors stay in one pixel, but a record whose detectors fall in different pixels takes
+// two entries, so pairs whose partners point apart are better kept as one row per detector.
 static void build_crossings(tb_obs *obs, cudaStream_t st) {
     if (obs->xrec) cudaFree(obs->xrec);
     if (obs->xqu) cudaFree(obs->xqu);
@@ -1223,24 +1339,31 @@ static void build_crossings(tb_obs *obs, cudaStream_t st) {
     obs->stable = nullptr;
     tb_free_blocked(obs);
     if (obs->lpix == nullptr || obs->V.total <= 0) return;
-    const int paired = obs->lpp != nullptr ? 1 : 0;
+    const bool intensity = obs->nnz == 1;
     const int64_t n_det = obs->d.n_det;
-    const int64_t n_rows = paired ? (n_det + 1) / 2 : n_det;
     const int64_t cpr = (obs->V.total + 31) / 32;
+    int paired = obs->lpp != nullptr ? 1 : 0;
+    std::vector<int32_t> hc;
+    if (intensity) {
+        paired = 0;
+        hc = count_crossings(obs, 0, n_det, cpr, nullptr, st);
+        if (n_det >= 2) {
+            int64_t split = 0, records_p = 0, entries_u = 0;
+            std::vector<int32_t> hp = count_crossings(obs, 1, (n_det + 1) / 2, cpr, &split, st);
+            for (int32_t c : hc) entries_u += c;
+            for (int32_t c : hp) records_p += c;
+            // (the 32-bit split counter is exact whenever the paired list can be built at all)
+            if (records_p < 2147483647LL && records_p + split < entries_u) {
+                paired = 1;
+                hc.swap(hp);
+            }
+        }
+    }
+    const int64_t n_rows = paired ? (n_det + 1) / 2 : n_det;
     const int64_t n_chunks = n_rows * cpr;
+    if (!intensity) hc = count_crossings(obs, paired, n_rows, cpr, nullptr, st);
     ObsDev o = make_dev(obs, 0);
-    int32_t *counts = nullptr;
-    TB_CUDA(cudaMalloc(&counts, sizeof(int32_t) * n_chunks));
     int grid = tbr::sm_count() * 8;
-    k_xbuild<false><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, counts, nullptr, nullptr,
-                                               nullptr);
-    TB_CUDA(cudaGetLastError());
-    tbr::count_launch();
-    std::vector<int32_t> hc(n_chunks);
-    TB_CUDA(cudaMemcpyAsync(hc.data(), counts, sizeof(int32_t) * n_chunks, cudaMemcpyDeviceToHost,
-                            st));
-    TB_CUDA(cudaStreamSynchronize(st));
-    cudaFree(counts);
     std::vector<int64_t> hb(n_chunks);
     std::vector<int64_t> row_ptr(n_rows + 1);
     int64_t total = 0;
@@ -1252,17 +1375,24 @@ static void build_crossings(tb_obs *obs, cudaStream_t st) {
         }
     }
     row_ptr[n_rows] = total;
-    // worth it only when the records are a smaller stream than the per-sample form
+    // worth it only when the records are a smaller stream than the per-sample form (intensity:
+    // a 16-byte record replaces at least one 17-byte stored sample)
     const double per_sample = (paired ? 12.0 : 20.0) * (double)obs->V.total * (double)n_det;
-    if (total == 0 || total >= 2147483647LL || 32.0 * (double)total > 0.8 * per_sample) return;
+    if (total == 0 || total >= 2147483647LL) return;
+    if (!intensity && 32.0 * (double)total > 0.8 * per_sample) return;
     int64_t *base = nullptr;
     TB_CUDA(cudaMalloc(&base, sizeof(int64_t) * n_chunks));
     TB_CUDA(cudaMemcpyAsync(base, hb.data(), sizeof(int64_t) * n_chunks, cudaMemcpyHostToDevice,
                             st));
     TB_CUDA(cudaMalloc(&obs->xrec, sizeof(int4) * total));
-    TB_CUDA(cudaMalloc(&obs->xqu, sizeof(double2) * total));
-    k_xbuild<true><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, nullptr, base, obs->xrec,
-                                              obs->xqu);
+    if (intensity) {
+        k_xbuild<true, 1><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, nullptr, base,
+                                                     obs->xrec, nullptr);
+    } else {
+        TB_CUDA(cudaMalloc(&obs->xqu, sizeof(double2) * total));
+        k_xbuild<true, 3><<<grid, kThreads, 0, st>>>(o, paired, n_rows, cpr, nullptr, base,
+                                                     obs->xrec, obs->xqu);
+    }
     TB_CUDA(cudaGetLastError());
     tbr::count_launch();
     // CTA table, TIME-major like tile_of_block: tile k of every row, then tile k + 1, ... so that
@@ -1306,14 +1436,17 @@ int tb_obs_pack_pointing(tb_obs *obs, void *stream) {
                "map too large for 32-bit local pixel indices");
     if (obs->lpix == nullptr) {
         TB_CUDA(cudaMalloc(&obs->lpix, sizeof(int32_t) * total));
-        TB_CUDA(cudaMalloc(&obs->wqu, sizeof(double2) * total));
+        if (obs->nnz == 3) TB_CUDA(cudaMalloc(&obs->wqu, sizeof(double2) * total));
     }
     ObsDev o = make_dev(obs, 0);
     unsigned zero = 0;
     TB_CUDA(cudaMemcpyToSymbolAsync(g_pack_mismatch, &zero, sizeof(zero), 0,
                                     cudaMemcpyHostToDevice, (cudaStream_t)stream));
     int grid = tbr::sm_count() * 8;
-    k_pack_pointing<<<grid, kThreads, 0, (cudaStream_t)stream>>>(o, obs->lpix, obs->wqu);
+    if (obs->nnz == 1)
+        k_pack_pointing<1><<<grid, kThreads, 0, (cudaStream_t)stream>>>(o, obs->lpix, nullptr);
+    else
+        k_pack_pointing<3><<<grid, kThreads, 0, (cudaStream_t)stream>>>(o, obs->lpix, obs->wqu);
     TB_CUDA(cudaGetLastError());
     tbr::count_launch();
     unsigned bad = 0;
@@ -1330,6 +1463,9 @@ int tb_obs_pack_pointing(tb_obs *obs, void *stream) {
         cudaFree(obs->wqu);
         obs->lpix = nullptr;
         obs->wqu = nullptr;
+    } else if (obs->V.total > 0 && obs->nnz == 1) {
+        // intensity: no weights to relate within a pair, the crossing list picks its rows
+        build_crossings(obs, (cudaStream_t)stream);
     } else if (obs->V.total > 0) {
         // pair form: fit the per-pair weight rotation on the first in-interval sample, then
         // verify it on every sample while writing the paired pixel records

@@ -122,6 +122,8 @@ PROTOTYPES = {
     "tb_cov_invert": (INT, [I64, I64, P, P, F64, INT, P]),
     "tb_obs_create": (P, [ct.POINTER(tb_obs_desc)]),
     "tb_obs_create_wcs": (P, [ct.POINTER(tb_obs_desc), ct.POINTER(tb_wcs_desc)]),
+    "tb_obs_create_intensity": (P, [ct.POINTER(tb_obs_desc), ct.POINTER(tb_wcs_desc)]),
+    "tb_obs_nnz": (INT, [P]),
     "tb_obs_destroy": (None, [P]),
     "tb_lhs_pass1": (INT, [P, P, P, P, INT, P]),
     "tb_lhs_pass2": (INT, [P, P, P, P, P, INT, P]),

@@ -152,14 +152,16 @@ class TemplateMatrix(Operator):
 
 class MapMaker(Operator):
     """Generalised destriper restricted to what the hot path covers: HEALPix
-    (``ops.PixelsHealpix``) or flat-sky WCS (``ops.PixelsWCS``) pointing, I/Q/U weights, a
-    diagonal noise model and ONE ``templates.Offset`` template.  With ``PixelsWCS`` the projection
+    (``ops.PixelsHealpix``) or flat-sky WCS (``ops.PixelsWCS``) pointing, I/Q/U or intensity-only
+    weights (``StokesWeights`` mode "IQU" or "I"), a diagonal noise model and ONE
+    ``templates.Offset`` template.  With ``PixelsWCS`` the projection
     is set up as that operator does (auto bounds from the boresights of every observation), and
     the pixel distribution carries ``wcs`` / ``wcs_shape``.
 
     Products placed in ``data`` (names as in ``ops/mapmaker.py:382-651``):
     ``{name}_hits``, ``{name}_cov``, ``{name}_rcond``, ``{name}_binmap`` (raw binned map),
-    ``{name}_map`` (template-cleaned map) and the solved ``AmplitudesMap`` under
+    ``{name}_map`` (template-cleaned map; 3 values per pixel, 1 in mode "I", whose covariance
+    has 1 value and whose rcond is 1 everywhere, as the reference sets it) and the solved ``AmplitudesMap`` under
     ``template_matrix.amplitudes``.  ``self.history`` is the PCG relative-residual history the
     reference logs at ``mapmaker_solve.py:701-706``.
     """
@@ -187,8 +189,10 @@ class MapMaker(Operator):
         pixels, weights = binning.pixel_pointing, binning.stokes_weights
         if pixels is None or weights is None:
             raise RuntimeError("binning must have pixel_pointing and stokes_weights set")
-        if weights.mode != "IQU":
-            raise NotImplementedError("the fused destriper implements mode='IQU'")
+        if weights.mode not in ("IQU", "I"):
+            raise NotImplementedError("the fused destriper implements mode='IQU' and mode='I'")
+        nnz = 3 if weights.mode == "IQU" else 1
+        ncov = nnz * (nnz + 1) // 2
         tmpls = self.template_matrix.templates
         if len(tmpls) != 1 or not isinstance(tmpls[0], Offset):
             raise NotImplementedError("MapMaker on the B200 path supports one Offset template")
@@ -268,7 +272,7 @@ class MapMaker(Operator):
                 hwp=ob.shared[weights.hwp_angle] if weights.hwp_angle is not None else None,
                 amp_offsets=np.array([tmpl._obs_amp_offset(x, iob) for x in dets],
                                      dtype=np.int64),
-                device=dev, **pixelisation)
+                nnz=nnz, device=dev, **pixelisation)
             dobs.append(d)
             # the timestreams are not needed before the RHS: their upload (the largest transfer)
             # runs on its own stream, underneath the pointing expansion, the covariance and the
@@ -306,17 +310,17 @@ class MapMaker(Operator):
 
         def covariance(threshold, want_hits):
             hmap = torch.zeros(n_loc * nps, dtype=torch.int64, device=dev) if want_hits else None
-            inv = torch.zeros((n_loc, nps, 6), dtype=torch.float64, device=dev)
+            inv = torch.zeros((n_loc, nps, ncov), dtype=torch.float64, device=dev)
             for d in dobs:
                 idx = np.arange(d.n_det, dtype=np.int32)
-                KC.cov_accum(dist.global_submap_to_local, n_loc, nps, 3, hmap, inv, idx, d.pixels,
+                KC.cov_accum(dist.global_submap_to_local, n_loc, nps, nnz, hmap, inv, idx, d.pixels,
                              idx, d.weights, idx, d.solver_flags, d.det_scale, 1, d.intervals,
                              None, 0)
             if hmap is not None:
                 allreduce_dev(hmap)
             allreduce_dev(inv)
             rc = torch.zeros(n_loc * nps, dtype=torch.float64, device=dev)
-            KC.cov_invert(n_loc * nps, 3, inv, rc, float(threshold))
+            KC.cov_invert(n_loc * nps, nnz, inv, rc, float(threshold))
             return hmap, inv, rc
 
         hmap, cov, rcond = covariance(self.solve_rcond_threshold, True)
@@ -326,14 +330,17 @@ class MapMaker(Operator):
         base_flags = [d.solver_flags.clone() for d in dobs]
 
         # rcond mask -> solver flags (mapmaker_templates.py:895-939 via ScanMask)
-        bad = torch.zeros((n_loc, nps, 3), dtype=torch.float64, device=dev)
+        bad = torch.zeros((n_loc, nps, nnz), dtype=torch.float64, device=dev)
         bad[:, :, 0] = (rcond.reshape(n_loc, nps) == 0).to(torch.float64)
         for d in dobs:
             idx = np.arange(d.n_det, dtype=np.int32)
             tmp = torch.zeros((d.n_det, d.n_samp), dtype=torch.float64, device=dev)
             # I weight may differ from 1 (cal): scan with unit weights on the first component
-            w1 = torch.zeros((d.n_det, d.n_samp, 3), dtype=torch.float64, device=dev)
-            w1[:, :, 0] = 1.0
+            if nnz == 3:
+                w1 = torch.zeros((d.n_det, d.n_samp, 3), dtype=torch.float64, device=dev)
+                w1[:, :, 0] = 1.0
+            else:
+                w1 = torch.ones((d.n_det, d.n_samp), dtype=torch.float64, device=dev)
             KC.ops_scan_map_float64(dist.global_submap_to_local, nps, bad, tmp, idx, d.pixels, idx,
                                     w1, idx, d.intervals, 1.0, True, False, False)
             d.solver_flags |= (tmp != 0).to(torch.uint8)
@@ -404,10 +411,10 @@ class MapMaker(Operator):
             return _pixdata_from_device(dist, t, dtype, nv)
 
         data[f"{self.name}_hits"] = to_pixdata(hmap, np.int64, 1)
-        data[f"{self.name}_cov"] = to_pixdata(ds.cov, np.float64, 6)
+        data[f"{self.name}_cov"] = to_pixdata(ds.cov, np.float64, ncov)
         data[f"{self.name}_rcond"] = to_pixdata(rcond_map, np.float64, 1)
-        data[f"{self.name}_binmap"] = to_pixdata(binmap, np.float64, 3)
-        data[f"{self.name}_map"] = to_pixdata(destriped, np.float64, 3)
+        data[f"{self.name}_binmap"] = to_pixdata(binmap, np.float64, nnz)
+        data[f"{self.name}_map"] = to_pixdata(destriped, np.float64, nnz)
         amps = AmplitudesMap()
         amps[tmpl.name] = tmpl.zeros()
         amps[tmpl.name].local[:] = amps_dev.cpu().numpy()

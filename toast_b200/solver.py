@@ -46,17 +46,22 @@ class DeviceObservation:
     layout (``templates/offset/offset.py:245-253``: detector-major, ceil(len/step) per view).
 
     The pixelisation is HEALPix (``nside`` / ``nest``) or a flat projection (``wcs``, a
-    ``toast_b200.wcs.FlatWCS`` with its shape set), one or the other."""
+    ``toast_b200.wcs.FlatWCS`` with its shape set), one or the other.  ``nnz`` is the number of
+    Stokes values per pixel: 3 (``StokesWeights(mode="IQU")``, weights [n_det, n_samp, 3]) or 1
+    (``mode="I"``, weights [n_det, n_samp] equal to ``cal[det]``)."""
 
     def __init__(self, *, focalplane, boresight, intervals, det_scale, step_length, n_pix_submap,
                  n_submap, global2local, nside=None, nest=None, wcs=None, amp_offset=0,
                  epsilon=None, gamma=None, cal=None, IAU=False, shared_flags=None,
                  shared_flag_mask=0, solver_flags=None, solver_flag_mask=255, pixels=None,
-                 weights=None, hwp=None, amp_offsets=None, compact=True, device="cuda"):
+                 weights=None, hwp=None, amp_offsets=None, compact=True, nnz=3, device="cuda"):
         if wcs is not None and (nside is not None or nest is not None):
             raise ValueError("DeviceObservation takes either wcs or nside / nest, not both")
         if wcs is None and (nside is None or nest is None):
             raise ValueError("DeviceObservation needs nside and nest, or wcs")
+        if nnz not in (1, 3):
+            raise ValueError("DeviceObservation supports nnz = 3 (I, Q, U) or 1 (I)")
+        self.nnz = int(nnz)
         self.device = torch.device(device)
         self.lib = L.load()
         self.n_det = int(focalplane.shape[0])
@@ -108,25 +113,29 @@ class DeviceObservation:
     def expand_pointing(self, hit_submaps=None):
         """PointingDetectorSimple -> PixelsHealpix (or PixelsWCS) -> StokesWeights in one fused
         kernel; fills ``pixels`` / ``weights`` on the device and ORs the hit-submap mask (host
-        uint8)."""
+        uint8).  With nnz = 1 the fused kernel writes the pixels only and StokesWeights(mode="I")
+        fills the [n_det, n_samp] weights."""
         dev = self.device
         if self.pixels is None:
             self.pixels = torch.zeros((self.n_det, self.n_samp), dtype=torch.int64, device=dev)
         if self.weights is None:
-            self.weights = torch.zeros((self.n_det, self.n_samp, 3), dtype=torch.float64,
-                                       device=dev)
+            shape = (self.n_det, self.n_samp, 3) if self.nnz == 3 else (self.n_det, self.n_samp)
+            self.weights = torch.zeros(shape, dtype=torch.float64, device=dev)
         idx = np.arange(self.n_det, dtype=np.int32)
+        fused_weights = self.weights if self.nnz == 3 else None
         if self.wcs is not None:
             K.pointing_fused_wcs(self.wcs, self.focalplane, self.boresight, self.shared_flags,
                                  self.shared_flag_mask, None, None, idx, self.pixels, idx,
-                                 self.weights, self.hwp, self.intervals, hit_submaps,
+                                 fused_weights, self.hwp, self.intervals, hit_submaps,
                                  self.n_pix_submap, self.epsilon, self.gamma, self.cal, self.IAU)
         else:
             K.pointing_fused(self.focalplane, self.boresight, self.shared_flags,
                              self.shared_flag_mask, None, None, idx, self.pixels, idx,
-                             self.weights, self.hwp, self.intervals, hit_submaps,
+                             fused_weights, self.hwp, self.intervals, hit_submaps,
                              self.n_pix_submap, self.nside, self.nest, self.epsilon, self.gamma,
                              self.cal, self.IAU)
+        if self.nnz == 1:
+            K.stokes_weights_I(idx, self.weights, self.intervals, self.cal)
         self._handle = None
 
     def set_global2local(self, g2l):
@@ -167,8 +176,11 @@ class DeviceObservation:
         d.pixels = L.ptr(self.pixels)
         d.weights = L.ptr(self.weights)
         d.hwp = L.ptr(self.hwp)
-        if self.wcs is not None:
-            self._wcs_desc = self.wcs.desc()
+        self._wcs_desc = self.wcs.desc() if self.wcs is not None else None
+        if self.nnz == 1:
+            h = self.lib.tb_obs_create_intensity(
+                ct.byref(d), ct.byref(self._wcs_desc) if self._wcs_desc is not None else None)
+        elif self.wcs is not None:
             h = self.lib.tb_obs_create_wcs(ct.byref(d), ct.byref(self._wcs_desc))
         else:
             h = self.lib.tb_obs_create(ct.byref(d))
@@ -183,7 +195,7 @@ class DeviceObservation:
         return bool(self.lib.tb_obs_has_compact_pointing(self.handle().h))
 
     def bytes_per_sample_stored(self):
-        return 8 + 24 + (1 if self.solver_flags is not None else 0)
+        return 8 + 8 * self.nnz + (1 if self.solver_flags is not None else 0)
 
 
 class _ObsHandle:
@@ -364,13 +376,20 @@ def pipeline_chunk_bounds(n_pix, world, n_chunks, align=1):
 class Destriper:
     """Fused SolverRHS / SolverLHS / solve() for one or more device observations.
 
-    ``cov`` is the inverse-of-inverse pixel covariance [n_local_submap, n_pix_submap, 6]
-    (upper triangle, row-major) as produced by ``covariance_invert``; ``regen=True``
-    recomputes pointing inside every pass instead of reading stored pixels/weights."""
+    ``cov`` is the inverse-of-inverse pixel covariance [n_local_submap, n_pix_submap,
+    nnz (nnz + 1) / 2] (upper triangle, row-major) as produced by ``covariance_invert``, with nnz
+    that of the observations (all the same: 3, or 1 for intensity-only maps); ``regen=True``
+    recomputes pointing inside every pass instead of reading stored pixels/weights.  Intensity
+    maps on several ranks are reduced with NCCL: the peer-memory reduction and the chunk pipeline
+    are IQU-only."""
 
     def __init__(self, observations, n_local_submap, n_pix_submap, cov, offset_var, amp_flags,
                  regen=False, group=None, device="cuda", fused_reduce=True, prior=None):
         self.obs = list(observations)
+        nnzs = {o.nnz for o in self.obs} or {3}
+        if len(nnzs) != 1:
+            raise ValueError("the observations of one Destriper must all have the same nnz")
+        self.nnz = nnzs.pop()
         # templates.offset_prior.OffsetPrior or None: with a noise prior the LHS gains the
         # inverse amplitude covariance (offset.py:884-960) and the preconditioner becomes the
         # banded / Toeplitz solve (offset.py:962-1010)
@@ -396,7 +415,7 @@ class Destriper:
         # the fused reduction works in 256-pixel tiles: maps that are not a multiple of that
         # (nside_submap < 8 gives 12 / 48 / 192 pixels per submap) take the NCCL path
         aligned = n_pix % 256 == 0
-        if self.world > 1 and fused_reduce and aligned and \
+        if self.world > 1 and fused_reduce and aligned and self.nnz == 3 and \
                 _os.environ.get("TB_FUSED_REDUCE", "1") != "0":
             import warnings
 
@@ -431,7 +450,7 @@ class Destriper:
         if self.peer is not None:
             self.zmap = self.peer.tensor.view(self.n_local_submap, self.n_pix_submap, 3)
         else:
-            self.zmap = torch.zeros((self.n_local_submap, self.n_pix_submap, 3),
+            self.zmap = torch.zeros((self.n_local_submap, self.n_pix_submap, self.nnz),
                                     dtype=torch.float64, device=self.device)
         # Chunk pipeline (multi-GPU): TB_PIPE_CHUNKS = "auto" (default: set it up with 4 chunks,
         # time it against the serial LHS on this node and keep the faster form), 0 (off) or K.
@@ -669,7 +688,7 @@ class Destriper:
             self.peer.reduce_cov(self.cov, stream=self._st())
             return
         self._allreduce(self.zmap)
-        L.check(self.lib.tb_cov_apply_diag(self.n_local_submap, self.n_pix_submap, 3,
+        L.check(self.lib.tb_cov_apply_diag(self.n_local_submap, self.n_pix_submap, self.nnz,
                                            L.ptr(self.cov), L.ptr(self.zmap), L.TB_MEM_DEVICE,
                                            self._st()))
 
