@@ -457,8 +457,11 @@ int tb_peer_set_multimem(int on); /* A/B switch: 0 = P2P kernel even when multic
 
 /* ---- a12/a13  amplitude-vector arithmetic for the PCG loop (templates/amplitudes.py:201-274,
  * :523-571; ops/mapmaker_solve.py:665-746).  All DEVICE pointers; scalars live on the device
- * so an iteration needs no host round trip.                                                 */
-/* out[0] = sum_{flags==0} a*b  (deterministic two-stage reduction) */
+ * so an iteration needs no host round trip.  n < 0, a NULL scalar pointer (delta, dq, out,
+ * sums) or a NULL vector when n > 0 (tb_amp_dot's flags excepted) is refused with TB_ERR_ARG
+ * before anything is launched.                                                              */
+/* out[0] = sum_{flags==0} a*b, every entry when flags is NULL (deterministic two-stage
+ * reduction) */
 int tb_amp_dot(const double *a, const double *b, const uint8_t *flags, int64_t n,
                double *out, void *stream);
 /* alpha = delta[0]/dq[0];  x += alpha d;  r -= alpha q;  s = flag ? 0 : r*var;

@@ -1614,6 +1614,9 @@ int tb_amp_dot(const double *a, const double *b, const uint8_t *flags, int64_t n
                void *stream) {
     TB_API_BEGIN
     tbr::require_device();
+    TB_REQUIRE(n >= 0, "negative vector length");
+    // flags may be NULL (every entry counts); the vectors may be NULL only when empty
+    TB_REQUIRE(out && (n == 0 || (a && b)), "NULL argument");
     RedScratch &r = red_scratch();
     k_amp_dot<<<red_grid(n), kThreads, 0, (cudaStream_t)stream>>>(a, b, flags, n, r.partials,
                                                                    r.counter, out);
@@ -1627,6 +1630,10 @@ int tb_pcg_update(const double *delta, const double *dq, double *x, double *r, c
                   int64_t n, double *sums, void *stream) {
     TB_API_BEGIN
     tbr::require_device();
+    TB_REQUIRE(n >= 0, "negative vector length");
+    // every thread reads the two scalars; the vectors may be NULL only when empty
+    TB_REQUIRE(delta && dq && sums && (n == 0 || (x && r && d && q && s && offset_var && flags)),
+               "NULL argument");
     RedScratch &rs = red_scratch();
     k_pcg_update<<<red_grid(n), kThreads, 0, (cudaStream_t)stream>>>(
         delta, dq, x, r, d, q, s, offset_var, flags, n, rs.partials, rs.counter, sums);
@@ -1639,6 +1646,8 @@ int tb_pcg_direction(const double *delta_new, const double *delta_old, double *d
                      int64_t n, void *stream) {
     TB_API_BEGIN
     tbr::require_device();
+    TB_REQUIRE(n >= 0, "negative vector length");
+    TB_REQUIRE(delta_new && delta_old && (n == 0 || (d && s)), "NULL argument");
     k_pcg_direction<<<red_grid(n), kThreads, 0, (cudaStream_t)stream>>>(delta_new, delta_old, d, s,
                                                                          n);
     TB_CUDA(cudaGetLastError());
