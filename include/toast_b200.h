@@ -377,6 +377,14 @@ int tb_bx_pass2(const tb_obs *obs, const double *binned, double *amplitudes_out,
                 void *stream);
 int tb_bx_fused(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_flags,
                 const double *cov, double *zmap_scratch, double *amplitudes_out, void *stream);
+/* The PCG's next direction (as tb_pcg_direction) with the prescale of the new d for the next
+ * tb_bx_fused(amplitudes = NULL) and q zeroed for its output, in one pass over d:
+ *   d = s + beta d (beta = delta_new[0] / delta_old[0]);  q = 0;  then delta_old[0] = delta_new[0].
+ * n must be the observation's whole amplitude vector, amp_offsets[det] = det * n_amp_det (what
+ * one observation on one GPU has); any other layout is refused with TB_ERR_ARG. */
+int tb_bx_direction_prescale(const tb_obs *obs, const double *delta_new, double *delta_old,
+                             double *d, const double *s, const uint8_t *amp_flags, double *q,
+                             int64_t n, void *stream);
 /* RHS projection (SolverRHS, mapmaker_solve.py:107-229): out += F^T N^-1 (signal - P m). */
 int tb_rhs_project(const tb_obs *obs, const double *signal, const uint8_t *amp_flags,
                    const double *binned, double *amplitudes_out, int regen, void *stream);

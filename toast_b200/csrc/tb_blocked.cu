@@ -157,16 +157,69 @@ k_bx_prescale(int paired, int n_det, int64_t nad, const int64_t *__restrict__ am
     for (int64_t i = (int64_t)blockIdx.y * kThreads + threadIdx.x; i < nad;
          i += (int64_t)gridDim.y * kThreads) {
         const bool g0 = __ldg(aflags + o0 + i) == 0;
-        const double a0 = g0 ? __ldg(amps + o0 + i) * w0 : 0.0;
+        const double2 t0 = bx_scaled(g0, g0 ? __ldg(amps + o0 + i) : 0.0, w0);
         if (paired) {
             const bool g1 = has1 && __ldg(aflags + o1 + i) == 0;
-            const double a1 = g1 ? __ldg(amps + o1 + i) * w1 : 0.0;
+            const double2 t1 = bx_scaled(g1, g1 ? __ldg(amps + o1 + i) : 0.0, w1);
             double2 *dst = reinterpret_cast<double2 *>(ascaled) + 2 * ((int64_t)row * nad + i);
-            dst[0] = make_double2(a0, a1);
-            dst[1] = make_double2(g0 ? w0 : 0.0, g1 ? w1 : 0.0);
+            dst[0] = make_double2(t0.x, t1.x);
+            dst[1] = make_double2(t0.y, t1.y);
         } else {
-            reinterpret_cast<double2 *>(ascaled)[(int64_t)row * nad + i] =
-                make_double2(a0, g0 ? w0 : 0.0);
+            reinterpret_cast<double2 *>(ascaled)[(int64_t)row * nad + i] = t0;
+        }
+    }
+}
+
+// The PCG's next direction (k_pcg_direction) fused with the prescale of that direction for the
+// next LHS and the zero-fill of the LHS output, in one pass over the rows x baselines of
+// k_bx_prescale: d = d beta + s, ascaled from the new d, q = 0.  The rows must cover the
+// amplitude vector (tb_bx_direction_prescale checks it), so every entry of d is advanced once.
+// delta_old <- delta_new is stored by the last CTA to finish: every CTA reads delta_old (thread
+// 0, before its counter increment) ahead of that store.
+__global__ void __launch_bounds__(kThreads)
+k_pcg_direction_prescale(int paired, int n_det, int64_t nad, const int64_t *__restrict__ amp_offsets,
+                         const double *__restrict__ det_scale, const double *dnew, double *dold,
+                         double *__restrict__ d, const double *__restrict__ s,
+                         const uint8_t *__restrict__ aflags, double *__restrict__ q,
+                         double *__restrict__ ascaled, unsigned int *counter) {
+    __shared__ double beta_sh;
+    if (threadIdx.x == 0) beta_sh = dnew[0] / dold[0];
+    __syncthreads();
+    const double beta = beta_sh;
+    const int row = blockIdx.x;
+    const int d0 = paired ? 2 * row : row, d1 = d0 + 1;
+    const bool has1 = paired && d1 < n_det;
+    const int64_t o0 = __ldg(amp_offsets + d0), o1 = has1 ? __ldg(amp_offsets + d1) : 0;
+    const double w0 = __ldg(det_scale + d0), w1 = has1 ? __ldg(det_scale + d1) : 0.0;
+    for (int64_t i = (int64_t)blockIdx.y * kThreads + threadIdx.x; i < nad;
+         i += (int64_t)gridDim.y * kThreads) {
+        const double n0 = pcg_direction(d[o0 + i], beta, s[o0 + i]);
+        d[o0 + i] = n0;
+        q[o0 + i] = 0.0;
+        const bool g0 = __ldg(aflags + o0 + i) == 0;
+        const double2 t0 = bx_scaled(g0, n0, w0);
+        if (paired) {
+            bool g1 = false;
+            double n1 = 0.0;
+            if (has1) {
+                n1 = pcg_direction(d[o1 + i], beta, s[o1 + i]);
+                d[o1 + i] = n1;
+                q[o1 + i] = 0.0;
+                g1 = __ldg(aflags + o1 + i) == 0;
+            }
+            const double2 t1 = bx_scaled(g1, n1, w1);
+            double2 *dst = reinterpret_cast<double2 *>(ascaled) + 2 * ((int64_t)row * nad + i);
+            dst[0] = make_double2(t0.x, t1.x);
+            dst[1] = make_double2(t0.y, t1.y);
+        } else {
+            reinterpret_cast<double2 *>(ascaled)[(int64_t)row * nad + i] = t0;
+        }
+    }
+    if (threadIdx.x == 0) {
+        __threadfence();
+        if (atomicAdd(counter, 1u) == gridDim.x * gridDim.y - 1) {
+            dold[0] = dnew[0];
+            *counter = 0u;
         }
     }
 }
@@ -548,6 +601,18 @@ void launch_bx_prescale(const tb_obs *obs, const double *amps, const uint8_t *af
     tbr::count_launch();
 }
 
+void launch_direction_prescale(const tb_obs *obs, const double *delta_new, double *delta_old,
+                               double *d, const double *s, const uint8_t *aflags, double *q,
+                               void *stream) {
+    dim3 grid;
+    row_grid(obs, grid);
+    k_pcg_direction_prescale<<<grid, kThreads, 0, (cudaStream_t)stream>>>(
+        obs->x_paired, (int)obs->d.n_det, obs->n_amp_det, obs->amp_offsets, obs->det_scale,
+        delta_new, delta_old, d, s, aflags, q, obs->ascaled, obs->bx_counter);
+    TB_CUDA(cudaGetLastError());
+    tbr::count_launch();
+}
+
 template <int MODE, int NNZ>
 void launch_bx_nnz(const tb_obs *obs, const BxArgs &a, int64_t n_units, void *stream) {
     const int64_t nb = (n_units + kBxWarps - 1) / kBxWarps;
@@ -618,7 +683,9 @@ void tb_free_blocked(tb_obs *obs) {
     if (obs->bunits_multi) cudaFree(obs->bunits_multi);
     if (obs->bmulti_blocks) cudaFree(obs->bmulti_blocks);
     if (obs->ascaled) cudaFree(obs->ascaled);
+    if (obs->bx_counter) cudaFree(obs->bx_counter);
     obs->ascaled = nullptr;
+    obs->bx_counter = nullptr;
     obs->brec = nullptr;
     obs->bqu = nullptr;
     obs->bunits = obs->bunits_single = obs->bunits_multi = nullptr;
@@ -693,6 +760,8 @@ void tb_build_blocked(tb_obs *obs, cudaStream_t st) {
             const size_t slots = (size_t)obs->n_xrows * (size_t)nad;
             const size_t per = obs->x_paired ? 2 : 1;
             TB_CUDA(cudaMalloc(&obs->ascaled, sizeof(double) * 2 * per * slots));
+            TB_CUDA(cudaMalloc(&obs->bx_counter, sizeof(unsigned int)));
+            TB_CUDA(cudaMemsetAsync(obs->bx_counter, 0, sizeof(unsigned int), st));
         }
         if (obs->nnz == 1)
             k_bx_gather<1><<<grid, kThreads, 0, st>>>(obs->xrec, nullptr, vout, n_sorted, nad, 1,
@@ -867,6 +936,22 @@ int tb_bx_fused(const tb_obs *obs, const double *amplitudes, const uint8_t *amp_
     a.cov = cov;
     a.out = amplitudes_out;
     launch_bx<2>(obs, a, obs->n_bunits_single, stream);
+    TB_API_END
+}
+
+int tb_bx_direction_prescale(const tb_obs *obs, const double *delta_new, double *delta_old,
+                             double *d, const double *s, const uint8_t *amp_flags, double *q,
+                             int64_t n, void *stream) {
+    TB_API_BEGIN
+    tbr::require_device();
+    TB_REQUIRE(obs && delta_new && delta_old && d && s && amp_flags && q, "NULL argument");
+    TB_REQUIRE(bx_ok(obs), "the observation has no block-ordered crossing list");
+    // one pass over the rows must reach every amplitude exactly once
+    const int64_t n_det = obs->d.n_det;
+    TB_REQUIRE(obs->amp_dense && n == n_det * obs->n_amp_det &&
+                   obs->n_xrows == (obs->x_paired ? (n_det + 1) / 2 : n_det),
+               "the crossing-list rows do not cover the amplitude vector");
+    launch_direction_prescale(obs, delta_new, delta_old, d, s, amp_flags, q, stream);
     TB_API_END
 }
 

@@ -176,4 +176,16 @@ __device__ __forceinline__ tbm::Quat detector_quat(const double *boresight, int6
     return tbm::qmul(b, fp);
 }
 
+// ---- PCG amplitude arithmetic ----------------------------------------------------------------
+// Shared by the separate kernels (k_pcg_direction, k_bx_prescale) and the fused one
+// (k_pcg_direction_prescale), which must leave the same bits.
+// next search direction: proposal *= beta; proposal += precond
+__device__ __forceinline__ double pcg_direction(double d, double beta, double s) {
+    return d * beta + s;
+}
+// one detector's entry of the prescaled amplitudes: {a w, w}, zeros for a flagged baseline
+__device__ __forceinline__ double2 bx_scaled(bool good, double a, double w) {
+    return make_double2(good ? a * w : 0.0, good ? w : 0.0);
+}
+
 } // namespace tbd

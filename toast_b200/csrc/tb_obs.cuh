@@ -31,6 +31,7 @@ struct tb_obs {
     // keep no (Q, U) arrays: wqu, xqu and bqu stay NULL, and lpp / pair_rot are never built.
     int nnz = 3;
     int64_t n_amp_det = 0;
+    int amp_dense = 0; // amp_offsets[det] == det * n_amp_det: the detectors tile [0, n_det n_amp_det)
     // compact solver pointing (tb_obs_pack_pointing): local pixel (int32, <0 = nothing to do)
     // and the two sample-dependent weights (Q, U) as one 16-byte record
     int32_t *lpix = nullptr;
@@ -51,6 +52,7 @@ struct tb_obs {
     // PIXEL BLOCK (kBxPix consecutive local pixels), i.e. in (block, row, time) order.  A CTA owns
     // one block at a time and keeps its 3 x kBxPix map values in shared memory.
     double *ascaled = nullptr;  // per-pass scratch [slot]{a0 w0, a1 w1, w0, w1} (k_bx_prescale)
+    unsigned int *bx_counter = nullptr; // k_pcg_direction_prescale: CTAs done (0 between launches)
     int2 *brec = nullptr;       // [n_brec] {pixel in block | n0 << kBxShift | n1 << (kBxShift+6), scaled-amplitude index}
     double2 *bqu = nullptr;     // [n_brec] (sum Q, sum U)
     int4 *bunits = nullptr;     // [n_bunits] {block, first record, end record, 1 if the block has several units}

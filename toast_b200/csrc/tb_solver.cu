@@ -1116,7 +1116,7 @@ k_pcg_direction(const double *__restrict__ dnew, const double *__restrict__ dold
     const double beta = dnew[0] / dold[0];
     for (int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x; i < n;
          i += (int64_t)gridDim.x * kThreads) {
-        d[i] = d[i] * beta + s[i]; // proposal *= beta; proposal += precond
+        d[i] = pcg_direction(d[i], beta, s[i]);
     }
 }
 
@@ -1205,6 +1205,9 @@ tb_obs *obs_create(const tb_obs_desc *desc, const tb_wcs_desc *wcs, int nnz) {
         o->gamma = dd + 6 * nd;
         o->det_scale = dd + 7 * nd;
         o->n_amp_det = acc;
+        o->amp_dense = 1;
+        for (int64_t i = 0; i < nd; ++i)
+            if (ib[3 * nv + 1 + i] != i * acc) o->amp_dense = 0;
         // the host arrays of the descriptor are not retained
         o->d.intervals = nullptr;
         o->d.epsilon = o->d.gamma = o->d.cal = o->d.det_scale = nullptr;

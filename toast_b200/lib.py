@@ -135,6 +135,7 @@ PROTOTYPES = {
     "tb_bx_pass1": (INT, [P, P, P, P, INT, I64, P]),
     "tb_bx_pass2": (INT, [P, P, P, I64, P]),
     "tb_bx_fused": (INT, [P, P, P, P, P, P, P]),
+    "tb_bx_direction_prescale": (INT, [P, P, P, P, P, P, P, I64, P]),
     "tb_rhs_project": (INT, [P, P, P, P, P, INT, P]),
     "tb_bin_signal": (INT, [P, P, P, INT, P]),
     "tb_offset_prior_create": (P, [ct.POINTER(tb_offset_prior_desc)]),

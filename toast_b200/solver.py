@@ -16,6 +16,9 @@ amplitude vectors of the PCG.  One iteration is
 with the scalars left on the device; the host reads back one float per iteration (the relative
 residual, which the reference logs at ``mapmaker_solve.py:701-706``) to test convergence.
 
+One observation on one GPU fuses the LHS into one kernel (tb_bx_fused), and the direction update
+also writes the prescaled d that kernel reads and zeroes q (tb_bx_direction_prescale).
+
 torch is used for device allocations and ``torch.distributed`` for the collectives only.
 """
 
@@ -458,6 +461,11 @@ class Destriper:
         # than serial with 8-16 (DESIGN.md section 5).
         # one observation on one GPU: pass 1 -> covariance -> pass 2 inside one kernel
         self.fuse_lhs = _os.environ.get("TB_FUSE_LHS", "1") != "0"
+        # (handle, d, q) whose prescaled d and zeroed q advance_direction left for the next LHS
+        self._prescaled = None
+        o = self.obs[0] if len(self.obs) == 1 else None
+        self._amps_tiled = o is not None and o.n_amp == self.n_amp and np.array_equal(
+            o.amp_offsets, np.arange(o.n_det, dtype=np.int64) * o.n_amp_det)
         self.pipeline = False
         self.blocked = False
         self.pipe_tune_ms = None
@@ -696,6 +704,7 @@ class Destriper:
         """This rank's raw noise-weighted map P^T N^-1 F a -- pass 1 only, no reduction, no
         covariance (diagnostics: bench.py checks the fused reduction against NCCL on it)."""
         st = torch.cuda.current_stream(self.device).cuda_stream
+        self._prescaled = None  # (pass 1 overwrites the prescaled amplitudes)
         if self._blocked():
             for k, o in enumerate(self.obs):
                 L.check(self.lib.tb_bx_pass1(o.handle().h, L.ptr(amps), L.ptr(self.amp_flags),
@@ -716,16 +725,32 @@ class Destriper:
         self.reduce_and_apply_cov()
         return self.zmap
 
+    def _fused_lhs(self):
+        """True when the LHS runs as the one fused kernel (one observation on one GPU)."""
+        return (self.world == 1 and len(self.obs) == 1 and self.fuse_lhs and not self.pipeline
+                and self._blocked())
+
+    def _direction_prescale(self):
+        """True when advance_direction can prescale the new direction for the fused LHS: the
+        fused LHS runs and the observation's detectors tile the whole amplitude vector."""
+        return self._amps_tiled and self._fused_lhs()
+
+    def _prescale_tag(self, d, q):
+        # tensor versions change with every in-place torch op: a d or q modified after
+        # advance_direction no longer matches its prescaled copy
+        return (self.obs[0].handle().h, d.data_ptr(), d._version, q.data_ptr(), q._version)
+
     def lhs(self, amps_in, amps_out, timers=None):
         """SolverLHS: amps_out = F^T N^-1 Z F amps_in.  ``timers``: optional list that receives
         four CUDA events (pass 1 start/end, pass 2 start/end) of the un-pipelined form."""
+        prescaled, self._prescaled = self._prescaled, None
         if self.pipeline and timers is None:
             self._lhs_pipelined(amps_in, amps_out)
             return self._add_prior(amps_in, amps_out)
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)] if timers is not None \
             else None
         if self._blocked():
-            return self._lhs_blocked(amps_in, amps_out, ev, timers)
+            return self._lhs_blocked(amps_in, amps_out, ev, timers, prescaled)
         self.zmap.zero_()
         if ev:
             ev[0].record()
@@ -747,23 +772,28 @@ class Destriper:
             timers.append(ev)
         return self._add_prior(amps_in, amps_out)
 
-    def _lhs_blocked(self, amps_in, amps_out, ev, timers):
+    def _lhs_blocked(self, amps_in, amps_out, ev, timers, prescaled=None):
         """The LHS on the block-ordered crossing list.  One observation on one GPU: ONE kernel
-        (pass 1 -> covariance -> pass 2 with the map tile in shared memory); otherwise pass 1
-        writes the map (no zero-fill, no atomics), the reduction + covariance follow, and pass 2
-        reads it back tile by tile."""
+        (pass 1 -> covariance -> pass 2 with the map tile in shared memory), which reuses the
+        prescaled amplitudes and the zeroed output advance_direction left when ``prescaled`` is
+        the tag of (amps_in, amps_out); otherwise pass 1 writes the map (no zero-fill, no
+        atomics), the reduction + covariance follow, and pass 2 reads it back tile by tile."""
         st = torch.cuda.current_stream(self.device).cuda_stream
         fused = self.world == 1 and len(self.obs) == 1 and self.fuse_lhs
-        amps_out.zero_()
+        reuse = fused and prescaled is not None and \
+            prescaled == self._prescale_tag(amps_in, amps_out)
+        if not reuse:
+            amps_out.zero_()
         if ev:
             ev[0].record()
         if fused:
             if ev:
                 ev[1].record()
                 ev[2].record()
-            L.check(self.lib.tb_bx_fused(self.obs[0].handle().h, L.ptr(amps_in),
-                                         L.ptr(self.amp_flags), L.ptr(self.cov), L.ptr(self.zmap),
-                                         L.ptr(amps_out), st))
+            L.check(self.lib.tb_bx_fused(self.obs[0].handle().h,
+                                         None if reuse else L.ptr(amps_in),
+                                         None if reuse else L.ptr(self.amp_flags), L.ptr(self.cov),
+                                         L.ptr(self.zmap), L.ptr(amps_out), st))
         else:
             for k, o in enumerate(self.obs):
                 L.check(self.lib.tb_bx_pass1(o.handle().h, L.ptr(amps_in), L.ptr(self.amp_flags),
@@ -839,6 +869,14 @@ class Destriper:
 
     def advance_direction(self, st):
         # delta_new = s.r = sums[1];  beta = delta_new / delta_old;  d = s + beta d
+        if self._direction_prescale():
+            # in the same pass: d prescaled for the fused LHS of (d, q), q zeroed, delta updated
+            L.check(self.lib.tb_bx_direction_prescale(
+                self.obs[0].handle().h, L.ptr(st.sums[1:]), L.ptr(st.delta), L.ptr(st.d),
+                L.ptr(st.s), L.ptr(self.amp_flags), L.ptr(st.q), self.n_amp, self._st()))
+            self._prescaled = self._prescale_tag(st.d, st.q)
+            return
+        self._prescaled = None
         L.check(self.lib.tb_pcg_direction(L.ptr(st.sums[1:]), L.ptr(st.delta), L.ptr(st.d),
                                           L.ptr(st.s), self.n_amp, self._st()))
         st.delta.copy_(st.sums[1:2])
