@@ -121,12 +121,13 @@ def _good_samples(pb, g2l, amp_offset=0):
     return det[good], lpix[good], amp[good]
 
 
-def _exact_sum(index, terms, n):
+def _exact_sum(index, terms, n, grain=DYADIC_GRAIN):
     """Per-index sums of `terms`, after checking that they cannot depend on summation order:
-    every term a multiple of 2^-16, and the sum of magnitudes of every index below 2^53 x 2^-16."""
-    assert np.all(np.mod(terms / DYADIC_GRAIN, 1.0) == 0.0), "a term is finer than 2^-16"
+    every term a multiple of `grain`, and the sum of magnitudes of every index below
+    2^53 x `grain`."""
+    assert np.all(np.mod(terms / grain, 1.0) == 0.0), f"a term is finer than {grain}"
     mag = np.bincount(index, weights=np.abs(terms), minlength=n)
-    assert np.max(mag, initial=0.0) / DYADIC_GRAIN < 2.0 ** 53, "a sum could round"
+    assert np.max(mag, initial=0.0) / grain < 2.0 ** 53, "a sum could round"
     return np.bincount(index, weights=terms, minlength=n)
 
 

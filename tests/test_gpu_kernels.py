@@ -231,25 +231,30 @@ def test_stokes_weights_I(K, ck):
 
 
 @pytest.mark.parametrize("name,n_det,n_samp", CASES)
-def test_pointing_fused_equals_chain(K, ck, name, n_det, n_samp):
+@pytest.mark.parametrize("hwp,IAU", [(False, False), (True, False), (False, True), (True, True)])
+def test_pointing_fused_equals_chain(K, ck, name, n_det, n_samp, hwp, IAU):
     obs = _obs(name, n_det, n_samp, eps_max=0.05)
     idx, q_ref = _quats(obs, ck)
     nside, nest = obs["nside"], obs["nest"]
     n_submap, nps = S.n_submap_for(nside, 16)
+    # a half-wave plate turning a few times a minute and a per-detector gamma
+    hwpang = (2.0 * np.pi * 3.0 / 60.0 / obs["rate"] * np.arange(n_samp)) % (2.0 * np.pi) \
+        if hwp else None
+    gamma = 0.3 * np.random.default_rng(4).random(n_det) if hwp else obs["gamma"]
     pix_ref = np.zeros((n_det, n_samp), dtype=np.int64)
     h_ref = np.zeros(n_submap, dtype=np.uint8)
     ck.pixels_healpix(idx, q_ref, obs["shared_flags"], 1, idx, pix_ref, obs["intervals"], h_ref,
                       nps, nside, nest, False)
     w_ref = np.zeros((n_det, n_samp, 3))
-    ck.stokes_weights_IQU(idx, q_ref, idx, w_ref, np.zeros(1), obs["intervals"], obs["epsilon"],
-                          obs["gamma"], obs["cal"], False, False)
+    ck.stokes_weights_IQU(idx, q_ref, idx, w_ref, np.zeros(1) if hwpang is None else hwpang,
+                          obs["intervals"], obs["epsilon"], gamma, obs["cal"], IAU, False)
     q = np.zeros_like(q_ref)
     pix = np.zeros_like(pix_ref)
     w = np.zeros_like(w_ref)
     h = np.zeros_like(h_ref)
     K.pointing_fused(obs["focalplane"], obs["boresight"], obs["shared_flags"], 1, idx, q, idx,
-                     pix, idx, w, None, obs["intervals"], h, nps, nside, nest, obs["epsilon"],
-                     obs["gamma"], obs["cal"], False, False)
+                     pix, idx, w, hwpang, obs["intervals"], h, nps, nside, nest, obs["epsilon"],
+                     gamma, obs["cal"], IAU, False)
     np.testing.assert_array_equal(q, q_ref)
     np.testing.assert_array_equal(pix, pix_ref)
     np.testing.assert_array_equal(h, h_ref)

@@ -77,6 +77,78 @@ def test_mapmaker_host_logic_with_oracle_compute(monkeypatch, name, n_det, n_sam
                       what="destriped map")
 
 
+@pytest.mark.parametrize("traits", ["cal", "hwp_IAU"])
+def test_stokes_weights_traits_reach_the_device(monkeypatch, traits):
+    """What StokesWeights computes the weights from must be what the device observation gets:
+    its `cal` key (ob[cal][det] overrides the focal plane's calibration, stokes_weights.py), its
+    half-wave-plate angle, IAU convention and the detectors' gamma.  The operator's products must
+    be the oracle's for the problem built with those inputs, and differ from the problem without
+    them."""
+    fake_device.install(monkeypatch)
+    obs = S.make_observation("c1", n_det=4, n_samp=6000, nside=64, eps_max=0.03)
+    rng = np.random.default_rng(5)
+    plain = dict(obs)
+    kw, wkw = {}, {}
+    if traits == "cal":
+        obs["cal"] = 0.75 + 0.5 * rng.random(obs["n_det"])
+        wkw = dict(cal="pointing_cal")
+    else:
+        obs["gamma"] = 0.3 * rng.random(obs["n_det"])
+        kw = dict(hwp=(np.arange(obs["n_samp"]) * 0.0123) % (2 * np.pi), IAU=True)
+        wkw = dict(hwp_angle="hwp_angle", IAU=True)
+    data = Data()
+    data.obs.append(observation_from_synthetic(plain if traits == "cal" else obs))
+    ob = data.obs[0]
+    if traits == "cal":
+        ob["pointing_cal"] = {d: float(c) for d, c in zip(ob.local_detectors, obs["cal"])}
+    else:
+        ob.shared["hwp_angle"] = kw["hwp"]
+    pb = O.build_problem(obs, O, rcond_threshold=1.0e-3, **kw)
+    pb_plain = O.build_problem(plain, O, rcond_threshold=1.0e-3)
+    dp = ops.PointingDetectorSimple(view="scanning", shared_flags="flags", shared_flag_mask=1)
+    pix = ops.PixelsHealpix(detector_pointing=dp, nside=obs["nside"], nest=obs["nest"],
+                            create_dist="pixel_dist")
+    wts = ops.StokesWeights(detector_pointing=dp, mode="IQU", **wkw)
+    binning = ops.BinMap(pixel_dist="pixel_dist", covariance="cov", pixel_pointing=pix,
+                         stokes_weights=wts, noise_model="noise_model", full_pointing=True)
+    tmpl = Offset(name="baselines", step_time=obs["step_time"], times="times",
+                  noise_model="noise_model")
+    tmat = ops.TemplateMatrix(templates=[tmpl], amplitudes="amplitudes")
+    mapper = ops.MapMaker(name="mm", det_data="signal", binning=binning, template_matrix=tmat,
+                          solve_rcond_threshold=1.0e-3, map_rcond_threshold=1.0e-3, iter_max=6,
+                          convergence=1.0e-30, device="cpu")
+    signal0 = obs["signal"].copy()
+    mapper.apply(data)
+    assert not np.array_equal(pb.cov, pb_plain.cov)
+    np.testing.assert_array_equal(data["mm_cov"].data, pb.cov)
+    np.testing.assert_array_equal(data["mm_binmap"].data,
+                                  O.bin_map(pb, O, signal0, O.cov_apply_diag))
+    rhs_ref = O.solver_rhs(pb, O, signal0)
+    amps_ref, hist_ref = O.solve(pb, O, rhs_ref, convergence=1e-30, n_iter_max=6)
+    assert mapper.history == hist_ref
+    np.testing.assert_array_equal(data["amplitudes"]["baselines"].local, amps_ref)
+
+
+def test_single_precision_weights_are_refused(monkeypatch):
+    fake_device.install(monkeypatch)
+    obs = S.make_observation("c1", n_det=2, n_samp=2000, nside=16)
+    data = Data()
+    data.obs.append(observation_from_synthetic(obs))
+    dp = ops.PointingDetectorSimple(view="scanning", shared_flags="flags", shared_flag_mask=1)
+    pix = ops.PixelsHealpix(detector_pointing=dp, nside=16, nest=obs["nest"],
+                            create_dist="pixel_dist")
+    wts = ops.StokesWeights(detector_pointing=dp, mode="IQU", single_precision=True)
+    binning = ops.BinMap(pixel_dist="pixel_dist", covariance="cov", pixel_pointing=pix,
+                         stokes_weights=wts, noise_model="noise_model", full_pointing=True)
+    tmat = ops.TemplateMatrix(templates=[Offset(name="baselines", step_time=obs["step_time"],
+                                                times="times", noise_model="noise_model")],
+                              amplitudes="amplitudes")
+    mapper = ops.MapMaker(name="mm", det_data="signal", binning=binning, template_matrix=tmat,
+                          iter_max=2, device="cpu")
+    with pytest.raises(NotImplementedError, match="single_precision"):
+        mapper.apply(data)
+
+
 def test_final_products_use_the_map_threshold_and_the_input_flags(monkeypatch):
     """ops/mapmaker.py:386-470, 502-594: the final covariance and maps are made with the binning
     flags (input flags, bad pointing, view) and map_rcond_threshold -- NOT with the solver's

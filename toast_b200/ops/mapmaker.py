@@ -191,6 +191,9 @@ class MapMaker(Operator):
             raise RuntimeError("binning must have pixel_pointing and stokes_weights set")
         if weights.mode not in ("IQU", "I"):
             raise NotImplementedError("the fused destriper implements mode='IQU' and mode='I'")
+        if weights.single_precision:
+            raise NotImplementedError("single_precision Stokes weights are not supported on the "
+                                      "B200 path")
         nnz = 3 if weights.mode == "IQU" else 1
         ncov = nnz * (nnz + 1) // 2
         tmpls = self.template_matrix.templates
@@ -240,6 +243,9 @@ class MapMaker(Operator):
         for iob, ob in enumerate(data.obs):
             dets = [d for d in tmpl._all_dets if d in tmpl._obs_dets[iob]]
             fp = ob[dp.focalplane_key]
+            # the Stokes weights' own focal plane and calibration, as StokesWeights._exec reads them
+            wfp = ob[weights.focalplane_key]
+            cal = [wfp[x]["cal"] if weights.cal is None else ob[weights.cal][x] for x in dets]
             # with a noise prior the baselines span the observation and the view only flags
             # samples (offset.py:136-141; the view flags are ORed into the solver flags below)
             iv = ob.intervals[tmpl._bounds_view if tmpl.use_noise_prior else view]
@@ -264,9 +270,9 @@ class MapMaker(Operator):
                 step_length=tmpl._step_length(tmpl.step_time, tmpl._obs_rate[iob]),
                 n_pix_submap=pixels._n_pix_submap, n_submap=pixels._n_submap,
                 global2local=np.zeros(pixels._n_submap, dtype=np.int64),
-                epsilon=np.array([fp[x]["epsilon"] for x in dets]),
-                gamma=np.array([fp[x]["gamma"] for x in dets]),
-                cal=np.array([fp[x]["cal"] for x in dets]), IAU=weights.IAU,
+                epsilon=np.array([wfp[x]["epsilon"] for x in dets]),
+                gamma=np.array([wfp[x]["gamma"] for x in dets]),
+                cal=np.array(cal, dtype=np.float64), IAU=weights.IAU,
                 shared_flags=ob.shared[dp.shared_flags] if dp.shared_flags is not None else None,
                 shared_flag_mask=dp.shared_flag_mask, solver_flags=flags, solver_flag_mask=1,
                 hwp=ob.shared[weights.hwp_angle] if weights.hwp_angle is not None else None,
