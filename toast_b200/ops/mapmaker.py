@@ -95,6 +95,57 @@ def _rows_from_device(dd, dets, t):
         dd.data[dd.indices(dets)] = t.cpu().numpy()
 
 
+class _SetUp:
+    """What one MapMaker call set up before its solve (device observations, pixel distribution,
+    covariances, flags, destriper); kept on the operator between calls with ``mc_mode=True``."""
+
+    def __init__(self, **kw):
+        self.__dict__.update(kw)
+
+    def update(self, **kw):
+        self.__dict__.update(kw)
+
+
+class _Same:
+    """Compares equal to a _Same of the very same object (whatever the object's own ``==``)."""
+
+    __slots__ = ("obj",)
+
+    def __init__(self, obj):
+        self.obj = obj
+
+    def __eq__(self, other):
+        return isinstance(other, _Same) and other.obj is self.obj
+
+    __hash__ = None
+
+
+_PLAIN = (type(None), bool, int, float, complex, str, bytes)
+
+
+def _setup_key(v):
+    """A snapshot of ``v`` that compares equal to a later snapshot when nothing the MapMaker
+    set-up reads from it has changed: plain values by value, arrays by content, operators and
+    templates (objects with ``_defaults``) by identity and the snapshots of their traits, anything
+    else by identity."""
+    if isinstance(v, _PLAIN):
+        return v
+    if isinstance(v, np.generic):
+        return v.item()
+    if isinstance(v, np.ndarray):
+        return ("ndarray", v.dtype.str, v.shape, v.tobytes())
+    if isinstance(v, (list, tuple)):
+        return tuple(_setup_key(x) for x in v)
+    if isinstance(v, dict):
+        return tuple((k, _setup_key(x)) for k, x in v.items())
+    traits = {}
+    for klass in reversed(type(v).__mro__):
+        traits.update(getattr(klass, "_defaults", {}))
+    if traits:
+        return (_Same(v), tuple((k, _setup_key(getattr(v, k, None))) for k in sorted(traits)))
+    return _Same(v)
+
+
 class TemplateMatrix(Operator):
     _defaults = dict(templates=None, amplitudes=None, transpose=False, view=None,
                      det_data="signal", det_mask=1, det_flags=None, det_flag_mask=1)
@@ -164,6 +215,24 @@ class MapMaker(Operator):
     has 1 value and whose rcond is 1 everywhere, as the reference sets it) and the solved ``AmplitudesMap`` under
     ``template_matrix.amplitudes``.  ``self.history`` is the PCG relative-residual history the
     reference logs at ``mapmaker_solve.py:701-706``.
+
+    ``mc_mode=True`` is for Monte Carlo runs, in which the same pointing, flags and noise weights
+    are destriped with one timestream after another (``mapmaker_templates.py:705-718,848-863``).
+    The first call runs the whole pipeline and keeps its set-up on the operator, on the device:
+    the device observations (expanded pointing, solver flags with the rcond mask, crossing lists
+    and compact pointing), the input flags of the final products, the pixel distribution, the
+    solve covariance (and the map covariance when ``map_rcond_threshold`` differs), the amplitude
+    flags and variance, the initialised Offset template with its noise prior, and the destriper.
+    A later call on the same ``Data`` with the same set-up traits uploads ``det_data``, solves
+    and bins the maps only: it replaces ``{name}_binmap``, ``{name}_map``, the amplitudes, the
+    cleaned timestream and ``history``, and leaves the first call's ``{name}_hits``,
+    ``{name}_cov`` and ``{name}_rcond`` in ``data``.  Flags are part of the set-up, as in the
+    reference: a realisation whose ``det_flags`` or shared flags differ from the first call's is
+    destriped with the first call's flags.  The set-up is rebuilt when the observations (or
+    their detectors or sample counts), the binning operator and its pointing, weights and noise
+    model, the template matrix and its template, the flag names and masks, the rcond thresholds,
+    ``regenerate_pointing``, ``device`` or ``det_mask`` change; on several ranks every rank
+    rebuilds when one does.  ``mc_mode=False`` drops what a previous call kept.
     """
 
     _defaults = dict(det_data="signal", det_mask=1, det_flags="flags", det_flag_mask=1,
@@ -171,12 +240,40 @@ class MapMaker(Operator):
                      iter_max=100, solve_rcond_threshold=1.0e-8, map_rcond_threshold=1.0e-8,
                      binning=None, template_matrix=None, map_binning=None,
                      regenerate_pointing=False, keep_solver_products=False, device="cuda",
-                     profile_stages=False)
+                     profile_stages=False, mc_mode=False)
+
+    def _mc_key(self, data, detectors):
+        """What the kept set-up was built from (see the class docstring)."""
+        tm = self.template_matrix
+        nm = self.binning.noise_model
+        observations = []
+        for ob in data.obs:
+            have = set(ob.detdata[self.det_data].detectors) if self.det_data in ob.detdata \
+                else set()
+            dets = tuple(d for d in ob.select_local_detectors(selection=detectors,
+                                                              flagmask=tm.det_mask)
+                         if d in have)
+            observations.append((_Same(ob), ob.n_local_samples, dets,
+                                 _Same(ob[nm] if nm in ob else None)))
+        traits = tuple((k, _setup_key(getattr(self, k))) for k in (
+            "binning", "template_matrix", "det_flags", "det_flag_mask", "shared_flags",
+            "shared_flag_mask", "solve_rcond_threshold", "map_rcond_threshold",
+            "regenerate_pointing", "device", "det_mask"))
+        return (_Same(data), tuple(observations), traits)
+
+    def _upload(self, ob, dets, dev, upload, main_stream):
+        """``det_data`` of ``dets`` to the device, on the ``upload`` stream."""
+        import torch
+
+        with torch.cuda.stream(upload):
+            sig = _rows_to_device(ob.detdata[self.det_data], dets, dev)
+        sig.record_stream(main_stream)
+        return sig
 
     def _exec(self, data, detectors=None, use_accel=True, **kwargs):
         import torch
 
-        from ..solver import DeviceObservation, Destriper
+        from ..solver import DeviceObservation, Destriper, _all_ranks_ok
 
         for trait in ("binning", "template_matrix"):
             if getattr(self, trait) is None:
@@ -230,6 +327,26 @@ class MapMaker(Operator):
             self.template_matrix.view
         self.template_matrix.det_data = self.det_data
         self.template_matrix.det_flags = None  # solver flags are applied on the device below
+        main_stream = torch.cuda.current_stream(dev)
+        upload = torch.cuda.Stream(device=dev)
+
+        # --- mc_mode: a later realisation on the kept set-up ------------------------------------
+        kept, self._mc_state = getattr(self, "_mc_state", None), None
+        if self.mc_mode:
+            reuse = kept is not None and kept.key == self._mc_key(data, detectors)
+            if comm.comm_world is not None:
+                # the set-up has collectives: every rank reuses or every rank rebuilds
+                reuse = _all_ranks_ok(reuse, dev)
+            if reuse:
+                signals = [self._upload(ob, dets, dev, upload, main_stream)
+                           for ob, dets in zip(data.obs, kept.dets)]
+                main_stream.wait_stream(upload)
+                mark("upload")
+                self._realise(data, kept, signals, mark, first=False)
+                self._mc_state = kept
+                return
+        del kept   # (a set-up that is not reused is freed before the next one is built)
+
         self.template_matrix.reset()
         tmpl._defer_prior = True  # built below, from the variance under the full solver flags
         tmpl._defer_variance = True  # (and so are the amplitude flags / variance themselves)
@@ -237,11 +354,10 @@ class MapMaker(Operator):
         self.template_matrix._init_templates(data, detectors)
 
         # --- device observations, solver flags bit 0 (mapmaker_templates.py:764-810) -----------
-        dobs, signals = [], []
-        main_stream = torch.cuda.current_stream(dev)
-        upload = torch.cuda.Stream(device=dev)
+        dobs, signals, obs_dets = [], [], []
         for iob, ob in enumerate(data.obs):
             dets = [d for d in tmpl._all_dets if d in tmpl._obs_dets[iob]]
+            obs_dets.append(dets)
             fp = ob[dp.focalplane_key]
             # the Stokes weights' own focal plane and calibration, as StokesWeights._exec reads them
             wfp = ob[weights.focalplane_key]
@@ -283,10 +399,7 @@ class MapMaker(Operator):
             # the timestreams are not needed before the RHS: their upload (the largest transfer)
             # runs on its own stream, underneath the pointing expansion, the covariance and the
             # construction of the crossing lists
-            with torch.cuda.stream(upload):
-                sig = _rows_to_device(ob.detdata[self.det_data], dets, dev)
-            sig.record_stream(main_stream)
-            signals.append(sig)
+            signals.append(self._upload(ob, dets, dev, upload, main_stream))
 
         mark("upload + flags")
         # --- pointing expansion + pixel distribution --------------------------------------------
@@ -310,26 +423,8 @@ class MapMaker(Operator):
 
         mark("pointing expansion")
         # --- CovarianceAndHits on the device (mapmaker_utils.py:1131-1270) ----------------------
-        def allreduce_dev(t):
-            if comm.comm_world is not None:
-                torch.distributed.all_reduce(t)
-
-        def covariance(threshold, want_hits):
-            hmap = torch.zeros(n_loc * nps, dtype=torch.int64, device=dev) if want_hits else None
-            inv = torch.zeros((n_loc, nps, ncov), dtype=torch.float64, device=dev)
-            for d in dobs:
-                idx = np.arange(d.n_det, dtype=np.int32)
-                KC.cov_accum(dist.global_submap_to_local, n_loc, nps, nnz, hmap, inv, idx, d.pixels,
-                             idx, d.weights, idx, d.solver_flags, d.det_scale, 1, d.intervals,
-                             None, 0)
-            if hmap is not None:
-                allreduce_dev(hmap)
-            allreduce_dev(inv)
-            rc = torch.zeros(n_loc * nps, dtype=torch.float64, device=dev)
-            KC.cov_invert(n_loc * nps, nnz, inv, rc, float(threshold))
-            return hmap, inv, rc
-
-        hmap, cov, rcond = covariance(self.solve_rcond_threshold, True)
+        st = _SetUp(dobs=dobs, dets=obs_dets, dist=dist, nnz=nnz, ncov=ncov, dev=dev, comm=comm)
+        hmap, cov, rcond = self._covariance(st, self.solve_rcond_threshold, True)
         # flags of the final products: the input flags only.  The solver's rcond mask (below) is
         # NOT part of them (ops/mapmaker.py:386-470, 502-594: the final covariance and maps are
         # made with the binning operator's own flags and map_rcond_threshold)
@@ -352,6 +447,8 @@ class MapMaker(Operator):
             d.solver_flags |= (tmp != 0).to(torch.uint8)
             del w1, tmp
         del bad
+        # (mc_mode: what the solver flags are set back to before every later solve)
+        solve_flags = [d.solver_flags.clone() for d in dobs] if self.mc_mode else None
 
         mark("covariance + rcond mask")
         # --- amplitude flags / preconditioner: n_good = F^T (good-sample indicator) -------------
@@ -388,6 +485,52 @@ class MapMaker(Operator):
                        regen=self.regenerate_pointing, device=dev, prior=tmpl.prior())
         main_stream.wait_stream(upload)   # the timestreams have arrived
         mark("crossing lists + solver set-up")
+        st.update(ds=ds, cov=cov, cov_map=None, base_flags=base_flags, solve_flags=solve_flags,
+                  hmap=hmap, rcond=rcond)
+        del base_flags, solve_flags, hmap, cov, rcond
+        self._realise(data, st, signals, mark, first=True)
+        if self.mc_mode:
+            st.key = self._mc_key(data, detectors)
+            self._mc_state = st
+
+    def _covariance(self, st, threshold, want_hits):
+        """(hits, covariance, rcond) of the observations under their current solver flags."""
+        import torch
+
+        dist, dev, nnz = st.dist, st.dev, st.nnz
+        n_loc, nps = dist.n_local_submap, dist.n_pix_submap
+
+        def allreduce_dev(t):
+            if st.comm.comm_world is not None:
+                torch.distributed.all_reduce(t)
+
+        hmap = torch.zeros(n_loc * nps, dtype=torch.int64, device=dev) if want_hits else None
+        inv = torch.zeros((n_loc, nps, st.ncov), dtype=torch.float64, device=dev)
+        for d in st.dobs:
+            idx = np.arange(d.n_det, dtype=np.int32)
+            KC.cov_accum(dist.global_submap_to_local, n_loc, nps, nnz, hmap, inv, idx, d.pixels,
+                         idx, d.weights, idx, d.solver_flags, d.det_scale, 1, d.intervals,
+                         None, 0)
+        if hmap is not None:
+            allreduce_dev(hmap)
+        allreduce_dev(inv)
+        rc = torch.zeros(n_loc * nps, dtype=torch.float64, device=dev)
+        KC.cov_invert(n_loc * nps, nnz, inv, rc, float(threshold))
+        return hmap, inv, rc
+
+    def _realise(self, data, st, signals, mark, first):
+        """The work that depends on the timestream: RHS, PCG, the final binning and the products
+        that change with ``det_data``.  ``first``: the call that built the set-up ``st``, which
+        also writes the hits, covariance and rcond products."""
+        ds, dobs, dist, nnz = st.ds, st.dobs, st.dist, st.nnz
+        tmpl = self.template_matrix.templates[0]
+        if not first:
+            # the previous final binning left the input flags and the map covariance in place:
+            # the solve needs the flags with the rcond mask, which the crossing lists and compact
+            # pointing were built from, in the SAME buffers (no invalidate), and its covariance
+            for d, sf in zip(dobs, st.solve_flags):
+                d.solver_flags.copy_(sf)
+            ds.cov = st.cov
         rhs = ds.rhs(signals)
         mark("RHS")
         amps_dev, self.history = ds.solve(rhs, convergence=self.convergence,
@@ -395,14 +538,16 @@ class MapMaker(Operator):
 
         mark("PCG")
         # --- final products -------------------------------------------------------------------------
-        for d, bf in zip(dobs, base_flags):
+        for d, bf in zip(dobs, st.base_flags):
             d.solver_flags.copy_(bf)   # (same buffer the native handle points at)
-        del base_flags
+        if not self.mc_mode:
+            st.base_flags = None
         if self.map_rcond_threshold != self.solve_rcond_threshold:
-            _, cov_map, rcond_map = covariance(self.map_rcond_threshold, False)
-            ds.cov = cov_map
+            if st.cov_map is None:
+                _, st.cov_map, rcond_map = self._covariance(st, self.map_rcond_threshold, False)
+            ds.cov = st.cov_map
         else:
-            rcond_map = rcond  # (the solve covariance was accumulated with the same flags)
+            rcond_map = st.rcond  # (the solve covariance was accumulated with the same flags)
         binmap = ds.bin_signal(signals).clone()
         neg = -amps_dev
         for d, sig in zip(dobs, signals):
@@ -416,9 +561,11 @@ class MapMaker(Operator):
         def to_pixdata(t, dtype, nv):
             return _pixdata_from_device(dist, t, dtype, nv)
 
-        data[f"{self.name}_hits"] = to_pixdata(hmap, np.int64, 1)
-        data[f"{self.name}_cov"] = to_pixdata(ds.cov, np.float64, ncov)
-        data[f"{self.name}_rcond"] = to_pixdata(rcond_map, np.float64, 1)
+        if first:
+            data[f"{self.name}_hits"] = to_pixdata(st.hmap, np.int64, 1)
+            data[f"{self.name}_cov"] = to_pixdata(ds.cov, np.float64, st.ncov)
+            data[f"{self.name}_rcond"] = to_pixdata(rcond_map, np.float64, 1)
+            st.hmap = st.rcond = None   # (on the host now; not needed by later realisations)
         data[f"{self.name}_binmap"] = to_pixdata(binmap, np.float64, nnz)
         data[f"{self.name}_map"] = to_pixdata(destriped, np.float64, nnz)
         amps = AmplitudesMap()
@@ -426,8 +573,7 @@ class MapMaker(Operator):
         amps[tmpl.name].local[:] = amps_dev.cpu().numpy()
         data[self.template_matrix.amplitudes] = amps
         # the cleaned timestream is what the reference leaves in det_data (mapmaker.py:531-574)
-        for iob, (ob, d, sig) in enumerate(zip(data.obs, dobs, signals)):
-            dets = [x for x in tmpl._all_dets if x in tmpl._obs_dets[iob]]
+        for ob, dets, sig in zip(data.obs, st.dets, signals):
             _rows_from_device(ob.detdata[self.det_data], dets, sig)
         mark("products to host")
         if self.keep_solver_products:

@@ -890,6 +890,13 @@ class Destriper:
         -- are enqueued first, so on exit x and r are exactly the reference's."""
         dev = self.device
         n = self.n_amp
+        # a Destriper that solves again (MapMaker mc_mode) gets new PCG vectors, which may land on
+        # the addresses of the previous solve's with their version counters back at 0: neither
+        # the previous prescale tag nor a graph captured on the previous vectors (or covariance)
+        # may be taken for theirs.  prepare_lhs below captures the graphs again, on every rank.
+        self._prescaled = None
+        if getattr(self, "_graphs", None):
+            self._graphs = {}
         st = _PCGState(n, dev)
         if x0 is not None:
             st.x.copy_(x0)
